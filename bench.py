@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- DEM Mcells/s for slope -> D8 -> flow accumulation -> HAND -> GFI (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--rows R --cols C]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--rows R --cols C] [--dump-outputs DIR]
 
 A "step" is one pass of the whole chain over one synthetic hydrologically conditioned DEM
 (recipe dtb-synth-v1, generated and depression-filled on the device before timing).  At N=1 the
@@ -15,6 +15,10 @@ DEM is sharded into N contiguous row bands (configs[3]; "scaling": "strong").
   cpu_baseline : the oracle port (oracle/dt_oracle.c, OpenMP) on a bounded sample, rank 0, N=1
 
   verified : device-side identities of the timed result (csrc/verify.cu), summed over ranks
+
+--dump-outputs DIR (1 GPU) writes the seven rasters of the last timed step as DIR/<name>.npy, integer rasters as float64
+(exact) and the others as float32: whole when they fit in 60 MiB, else the same seeded sample of cells from every raster.
+The DEM depends only on --rows / --cols, so two builds run with the same arguments can be compared output for output.
 
 --impl reference times the reference's own CPU path on the host cores: the unmodified reference installed under
 baseline/_ref (pip --target, git-ignored, travels with the snapshot) through its compiled Numba CPU-jit twins
@@ -50,6 +54,7 @@ KERNEL_BYTES = {
 # what the dominant kernel cannot avoid moving through DRAM: table 2 + dem 4 in, four rasters 16 out (the dem[idx] / acc[idx]
 # gathers are resolved once per tile exit and served by L2)
 KERNEL_COMPULSORY_BYTES = {"hand_tile_kernel<table>": 22, "slope_d8_tma_kernel": 9, "fa_tile_kernel": 7}
+DUMP_BYTES, DUMP_SEED = 60 << 20, 0  # --dump-outputs: data bytes of all files (< 64 MB), seed of the sampled cells
 SAMPLE_ROWS = SAMPLE_COLS = 3072  # bounded CPU sample of the OpenMP port
 REF_SAMPLE = 1536                    # bounded sample of the single-threaded reference (about 1 s per step)
 GPU_REF_SAMPLE = 4096                # the reference's own Numba-CUDA kernels on the same GPU
@@ -291,6 +296,24 @@ def extra_kernels(peak):
     return out
 
 
+def dump_outputs(outs, path):
+    """--dump-outputs: the rasters in `outs` as path/<name>.npy (see the module docstring)"""
+    import numpy as np
+    import torch
+
+    wide = {k: torch.float64 if t.dtype in (torch.int32, torch.int64) else torch.float32 for k, t in outs.items()}
+    per_cell = sum(8 if d == torch.float64 else 4 for d in wide.values())
+    n = next(iter(outs.values())).numel()
+    cells = None
+    if n * per_cell > DUMP_BYTES:
+        rng = np.random.default_rng(DUMP_SEED)
+        cells = torch.from_numpy(np.unique(rng.integers(0, n, DUMP_BYTES // per_cell))).cuda()
+    os.makedirs(path, exist_ok=True)
+    for k, t in outs.items():
+        v = t if cells is None else t.reshape(-1)[cells]
+        np.save(os.path.join(path, k + ".npy"), v.to(wide[k]).cpu().numpy())
+
+
 def workload_name(args):
     cond = "not depression-filled" if getattr(args, "unconditioned", False) else "depression-filled"
     return f"synthetic {args.rows}x{args.cols} f32 DEM (dtb-synth-v1, {cond}), full slope->D8->flowacc->HAND->GFI chain"
@@ -308,6 +331,8 @@ def run_ours(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if world != args.gpus:
         raise SystemExit(f"--gpus {args.gpus} but WORLD_SIZE={world}: launch with torchrun --nproc-per-node {args.gpus}")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs is for one GPU")
     torch.cuda.set_device(local)
     from descriptools_b200 import bands as _bands
 
@@ -404,6 +429,8 @@ def run_ours(args):
                                  row0=runner.bands[0].r0, total_rows=rows)
         dist.all_reduce(cnt)
     verdict = device.chain_verdict(cnt.tolist())
+    if args.dump_outputs:
+        dump_outputs(outs, args.dump_outputs)
     ms = t_start.elapsed_time(t_end)
     for e in events:
         for i, k in enumerate(stage_ms):
@@ -590,7 +617,12 @@ def main():
     ap.add_argument("--unconditioned", action="store_true",
                     help="N>1 only: every rank synthesises its band, no depression filling (sizes no single GPU can condition)")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-API leg (pinned staging buffers may exceed host RAM)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the rasters of the last timed step to DIR/<name>.npy (1 GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

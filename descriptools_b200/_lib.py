@@ -16,6 +16,7 @@ DTB_F32, DTB_I16 = 0, 1
 DTB_I32, DTB_I64 = 0, 1
 DTB_FA_FULL, DTB_FA_SUMMARY, DTB_FA_FINISH = 0, 1, 2
 DTB_HAND_FULL, DTB_HAND_SUMMARY, DTB_HAND_FINISH = 0, 1, 2
+DTB_FILL_INIT, DTB_FILL_SOLVE = 0, 1
 
 
 class DtbError(RuntimeError):
@@ -151,6 +152,9 @@ SIGNATURES = {
                                   c_float, c_void_p, c_void_p]),
     "dtb_fill_workspace_bytes": (c_size_t, [c_int64, c_int64]),
     "dtb_fill_depressions_f32": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_size_t, POINTER(c_int), c_void_p]),
+    "dtb_fill_band_workspace_bytes": (c_size_t, [c_int64, c_int64]),
+    "dtb_fill_band_f32": (c_int, [c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_void_p, c_size_t, POINTER(c_int), POINTER(c_int),
+                                  c_void_p]),
 }
 
 

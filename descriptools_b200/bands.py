@@ -224,6 +224,7 @@ class Band:
         self.fa_inflow = torch.zeros((2, cols), dtype=i64, device=device)
         self.hand_sum = torch.zeros((8, cols), dtype=i64, device=device)
         self.hand_res = torch.zeros((8, cols), dtype=i64, device=device)
+        self.ws_fill = None  # depression filling only: allocated by fill_init, freed by fill_release
 
     # views
     @property
@@ -344,6 +345,77 @@ class Band:
 
     def outputs(self) -> dict:
         return dict(slope=self.slope, d8=self.d8, acc=self.acc, fdist=self.fdist, idx=self.idx, hand=self.hand, gfi=self.gfi)
+
+    # depression filling (fill_rounds): the (rows + 2) x cols view dem_buf[1:rows+3], one halo row per side
+    def fill_halo_items(self):
+        """(first row, last row, halo row above, halo row below) for the exchange's halo()"""
+        r = self.rows
+        return self.dem_buf[2], self.dem_buf[r + 1], self.dem_buf[1], self.dem_buf[r + 2]
+
+    def _fill(self, mode) -> tuple[int, int]:
+        passes, seam = ctypes.c_int(0), ctypes.c_int(0)
+        self._check(self.lib.dtb_fill_band_f32(self.dem_buf[1].data_ptr(), self.rows, self.cols, 0 if self.first else 1,
+                                               0 if self.last else 1, mode, self.ws_fill.data_ptr(), self.ws_fill.numel(),
+                                               ctypes.byref(passes), ctypes.byref(seam), self._stream()), "dtb_fill_band_f32")
+        return int(passes.value), int(seam.value)
+
+    def fill_init(self):
+        """halo rows = the neighbours' DEM rows: seed mask, then an upper bound of the fill written into the band.  The
+        workspace (5 bytes per cell: elevations + seed mask) lives until fill_release()."""
+        from ._lib import DTB_FILL_INIT
+
+        self.ws_fill = torch.empty(self.lib.dtb_fill_band_workspace_bytes(self.rows, self.cols), dtype=torch.uint8, device=self.dev)
+        self._fill(DTB_FILL_INIT)
+
+    def fill_solve(self) -> tuple[int, int]:
+        """halo rows = the neighbours' current seam rows: relax the band to its fixed point -> (passes, seam row lowered)"""
+        from ._lib import DTB_FILL_SOLVE
+
+        return self._fill(DTB_FILL_SOLVE)
+
+    def fill_release(self):
+        self.ws_fill = None
+
+
+# ---- depression filling over bands -------------------------------------------------------------------
+FILL_MAX_ROUNDS = 10000
+
+
+def fill_rounds(bands, x, max_rounds: int = FILL_MAX_ROUNDS) -> dict:
+    """Priority-flood+epsilon filling of the raster held by `bands` (this process's bands; `x` the exchange), bit-identical
+    to the single-raster fill (dtb_fill_depressions_f32).
+
+    The fill is the unique fixed point of W(c) = max(z(c), min over the 8 neighbours of succ(W(n))), and relaxing any
+    upper bound converges to it, so the bands relax block-Jacobi: every band starts from an upper bound built from its
+    own rows (fill_init), then each round exchanges the seam rows and every band relaxes to its own fixed point with its
+    halo rows held constant (fill_solve).  A round in which no band lowered a cell of its first or last row leaves every
+    band fixed under halos equal to its neighbours' current rows: the whole raster is then the fixed point.
+
+    A band is anything with fill_halo_items / fill_init / fill_solve / fill_release and a `dev` (tests pass NumPy
+    stand-ins).  Returns {"rounds": n, "passes": [relaxation passes of each local band]}."""
+    items = [b.fill_halo_items() for b in bands]
+    x.halo(items)  # the DEM rows next to the seams: a cell beside nodata across a seam is a seed
+    passes = [0] * len(bands)
+    try:
+        for b in bands:
+            b.fill_init()
+        for rnd in range(1, max_rounds + 1):
+            x.halo(items)
+            moved = 0
+            for k, b in enumerate(bands):
+                p, s = b.fill_solve()
+                passes[k] += p
+                moved += s
+            if isinstance(x, DistExchange):
+                t = torch.tensor([moved], dtype=torch.int64, device=bands[0].dev)
+                x.dist.all_reduce(t, group=x.group)
+                moved = int(t.item())
+            if moved == 0:
+                return {"rounds": rnd, "passes": passes}
+    finally:
+        for b in bands:
+            b.fill_release()
+    raise RuntimeError(f"depression filling over bands did not converge in {max_rounds} rounds")
 
 
 # ---- exchange back-ends ----------------------------------------------------------------------------
@@ -487,10 +559,18 @@ class BandRunner:
         for b, d in zip(self.bands, dem_rows):
             b.dem.copy_(d, non_blocking=True)
 
-    def load_file(self, path, decode: str = "auto", nodata=None):
+    def fill_depressions(self, max_rounds: int = FILL_MAX_ROUNDS) -> dict:
+        """Fill the depressions of the loaded DEM in place, band by band (fill_rounds): the result equals
+        device.fill_depressions on the whole raster, bit for bit, and no rank holds more than its band (plus a 5 bytes
+        per cell workspace for the duration of the call).  Returns {"rounds": n, "passes": [per local band]}."""
+        return fill_rounds(self.bands, self.x, max_rounds)
+
+    def load_file(self, path, decode: str = "auto", nodata=None, condition: bool = False):
         """Every local band decodes its own rows of a float32 DEM GeoTIFF straight into its device buffer
         (raster.read_to_device(rows=...): with decode="device" only the band's compressed tiles cross PCIe); the file's
-        nodata value (or `nodata`) becomes the path's sentinel -100, as example.py:42-43 does on the host."""
+        nodata value (or `nodata`) becomes the path's sentinel -100, as example.py:42-43 does on the host.
+        `condition=True` then fills the DEM's depressions over the bands (fill_depressions), for DEMs no GIS has
+        conditioned yet."""
         from . import raster
 
         with raster.open(path) as src:
@@ -504,6 +584,8 @@ class BandRunner:
 
                 raster.read_to_device(src, out=b.dem, rows=(b.r0, b.r1), decode=decode)
                 _device.nodata_to_sentinel(b.dem, nd)
+        if condition:
+            self.fill_depressions()
 
     def step(self, events=None, hook=None, check=True):
         """One pass of the chain; `events` (4 CUDA events) are recorded at the stage boundaries and `hook(i)` is

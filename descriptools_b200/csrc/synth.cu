@@ -147,9 +147,13 @@ fill_rowscan_kernel(const float *__restrict__ zsrc, const uint8_t *__restrict__ 
 constexpr int FT = 32;          // tile edge
 constexpr int TILE_ITERS = 24;  // in-tile sweeps per pass
 
-__global__ void __launch_bounds__(256)
-fill_relax_kernel(const float *__restrict__ zsrc, const uint8_t *__restrict__ fixed, int64_t rows, int64_t cols,
-                  float *w, int tiles_x, unsigned *__restrict__ changed)
+// One pass over one tile.  BAND: w points at row 0 of a band whose halo rows -1 / rows (the neighbours' current
+// seam rows) are read where the band has a neighbour -- as constants, never stored -- and *seam is set when a cell
+// of the band's first or last row is lowered.  The single-raster instantiation is the original kernel body.
+template <bool BAND>
+__device__ __forceinline__ void fill_relax_tile(const float *__restrict__ zsrc, const uint8_t *__restrict__ fixed, int64_t rows,
+                                                int64_t cols, float *w, int tiles_x, unsigned *__restrict__ changed,
+                                                int64_t row_lo, int64_t row_hi, unsigned *__restrict__ seam)
 {
     __shared__ float sw[FT + 2][FT + 3];
     const int ty = blockIdx.x / tiles_x, tx = blockIdx.x - ty * tiles_x;
@@ -159,7 +163,10 @@ fill_relax_kernel(const float *__restrict__ zsrc, const uint8_t *__restrict__ fi
         const int j = idx / (FT + 2), k = idx - j * (FT + 2);
         const int64_t r = r0 - 1 + j, c = c0 - 1 + k;
         float v = __int_as_float(0x7f800000);  // +inf outside: never the minimum
-        if (r >= 0 && r < rows && c >= 0 && c < cols) v = __ldcg(&w[r * cols + c]);
+        bool rin;
+        if constexpr (BAND) rin = r >= row_lo && r < row_hi;
+        else rin = r >= 0 && r < rows;
+        if (rin && c >= 0 && c < cols) v = __ldcg(&w[r * cols + c]);
         sw[j][k] = v;
     }
     float z[4];
@@ -172,7 +179,7 @@ fill_relax_kernel(const float *__restrict__ zsrc, const uint8_t *__restrict__ fi
         z[i] = in ? zsrc[r * cols + c] : 0.0f;
     }
     __syncthreads();
-    bool any = false;
+    bool any = false, edge = false;
     for (int it = 0; it < TILE_ITERS; ++it) {
         bool ch = false;
 #pragma unroll
@@ -182,7 +189,14 @@ fill_relax_kernel(const float *__restrict__ zsrc, const uint8_t *__restrict__ fi
             float m = fminf(fminf(sw[j - 1][k - 1], sw[j - 1][k]), fminf(sw[j - 1][k + 1], sw[j][k - 1]));
             m = fminf(m, fminf(fminf(sw[j][k + 1], sw[j + 1][k - 1]), fminf(sw[j + 1][k], sw[j + 1][k + 1])));
             const float v = fmaxf(z[i], succ(m));
-            if (v < sw[j][k]) { sw[j][k] = v; ch = true; }
+            if (v < sw[j][k]) {
+                sw[j][k] = v;
+                ch = true;
+                if constexpr (BAND) {
+                    const int64_t r = r0 + ly + 8 * i;
+                    edge |= r == 0 || r == rows - 1;
+                }
+            }
         }
         any |= ch;
         if (!__syncthreads_or(ch)) break;
@@ -193,6 +207,60 @@ fill_relax_kernel(const float *__restrict__ zsrc, const uint8_t *__restrict__ fi
             if (!fx[i]) __stcg(&w[(r0 + ly + 8 * i) * cols + c0 + lx], sw[ly + 8 * i + 1][lx + 1]);
     }
     if (__syncthreads_or(any) && threadIdx.x == 0) atomicAdd(changed, 1u);
+    if constexpr (BAND) {
+        if (__syncthreads_or(edge) && threadIdx.x == 0) atomicOr(seam, 1u);
+    }
+}
+
+__global__ void __launch_bounds__(256)
+fill_relax_kernel(const float *__restrict__ zsrc, const uint8_t *__restrict__ fixed, int64_t rows, int64_t cols,
+                  float *w, int tiles_x, unsigned *__restrict__ changed)
+{
+    fill_relax_tile<false>(zsrc, fixed, rows, cols, w, tiles_x, changed, 0, 0, nullptr);
+}
+
+// ---- depression filling over row bands ----------------------------------------------------------
+// A band's buffer is (rows + 2) x cols: rows 0 and rows + 1 are halo rows (the neighbours' rows next to the seams),
+// the kernels get w = row 1.  Block-Jacobi over bands: every band relaxes to its own fixed point with the halo rows
+// held constant; the driver exchanges the seam rows and repeats until no seam row changes (descriptools_b200/bands.py).
+
+// as fill_mask_kernel, but the top / bottom row is a seed only where the band has no neighbour; elsewhere the halo
+// row decides whether a cell touches nodata across the seam
+__global__ void __launch_bounds__(256)
+fill_band_mask_kernel(const float *__restrict__ w, int64_t rows, int64_t cols, int has_above, int has_below,
+                      float *__restrict__ zsrc, uint8_t *__restrict__ fixed)
+{
+    const int64_t n = rows * cols;
+    const int64_t p = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (p >= n) return;
+    const int64_t r = p / cols, c = p - r * cols;
+    const float z = w[p];
+    zsrc[p] = z;
+    bool fx = is_nd(z) || c == 0 || c == cols - 1 || (r == 0 && !has_above) || (r == rows - 1 && !has_below);
+    if (!fx) {  // rows -1 and `rows` are read only where the band has that neighbour
+#pragma unroll
+        for (int dr = -1; dr <= 1; ++dr)
+#pragma unroll
+            for (int dc = -1; dc <= 1; ++dc) fx |= is_nd(w[p + dr * cols + dc]);
+    }
+    fixed[p] = fx ? 1 : 0;
+}
+
+// a band below another one has no column of seeds above it: its non-seed cells start at +inf, and the row scan (every
+// row starts at the seed in column 0) brings them down to an upper bound
+__global__ void __launch_bounds__(256)
+fill_band_inf_kernel(const uint8_t *__restrict__ fixed, int64_t n, float *__restrict__ w)
+{
+    const int64_t p = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (p < n && !fixed[p]) w[p] = __int_as_float(0x7f800000);
+}
+
+__global__ void __launch_bounds__(256)
+fill_relax_band_kernel(const float *__restrict__ zsrc, const uint8_t *__restrict__ fixed, int64_t rows, int64_t cols,
+                       float *w, int tiles_x, unsigned *__restrict__ changed, int64_t row_lo, int64_t row_hi,
+                       unsigned *__restrict__ seam)
+{
+    fill_relax_tile<true>(zsrc, fixed, rows, cols, w, tiles_x, changed, row_lo, row_hi, seam);
 }
 
 }  // namespace
@@ -256,5 +324,66 @@ extern "C" int dtb_fill_depressions_f32(float *dem, int64_t rows, int64_t cols, 
         if (passes > kMaxPasses) return DTB_ERR_UNSUPPORTED;
     }
     if (iterations_host) *iterations_host = passes;
+    return DTB_OK;
+}
+
+// workspace layout as dtb_fill_workspace_bytes: flags (changed at byte 0, seam at byte 4), zsrc, fixed
+extern "C" size_t dtb_fill_band_workspace_bytes(int64_t rows, int64_t cols) { return dtb_fill_workspace_bytes(rows, cols); }
+
+extern "C" int dtb_fill_band_f32(float *dem_halo, int64_t rows, int64_t cols, int has_above, int has_below, int mode, void *ws,
+                                 size_t ws_bytes, int *passes_host, int *seam_changed_host, void *stream)
+{
+    if (!dem_halo || !ws || rows <= 0 || cols <= 0) return DTB_ERR_INVALID;
+    if ((has_above != 0 && has_above != 1) || (has_below != 0 && has_below != 1)) return DTB_ERR_INVALID;
+    if (mode != DTB_FILL_INIT && mode != DTB_FILL_SOLVE) return DTB_ERR_INVALID;
+    if (ws_bytes < dtb_fill_band_workspace_bytes(rows, cols)) return DTB_ERR_WORKSPACE;
+    const int tiles_x = (int)((cols + FT - 1) / FT);
+    const int64_t ntiles = (int64_t)tiles_x * ((rows + FT - 1) / FT);
+    if (ntiles > 0x7fffffff) return DTB_ERR_UNSUPPORTED;
+    cudaStream_t st = as_stream(stream);
+    const int64_t n = rows * cols;
+    unsigned *flags = reinterpret_cast<unsigned *>(ws);  // [0] a tile changed, [1] a seam row changed
+    float *zsrc = reinterpret_cast<float *>((char *)ws + 256);
+    uint8_t *fixed = reinterpret_cast<uint8_t *>((char *)ws + 256 + (size_t)n * 4);
+    float *w = dem_halo + cols;
+    int passes = 0;
+    unsigned seam = 0;
+    if (mode == DTB_FILL_INIT) {
+        const unsigned blocks = (unsigned)((n + 255) / 256);
+        fill_band_mask_kernel<<<blocks, 256, 0, st>>>(w, rows, cols, has_above, has_below, zsrc, fixed);
+        DTB_LAUNCH_CHECK("fill_band_mask_kernel");
+        if (!has_above) {  // the band holds the raster's top row: the column scan starts at its seeds
+            fill_colscan_kernel<<<(unsigned)((cols + 127) / 128), 128, 0, st>>>(zsrc, fixed, rows, cols, w);
+            DTB_LAUNCH_CHECK("fill_colscan_kernel");
+        } else {
+            fill_band_inf_kernel<<<blocks, 256, 0, st>>>(fixed, n, w);
+            DTB_LAUNCH_CHECK("fill_band_inf_kernel");
+        }
+        fill_rowscan_kernel<<<(unsigned)((rows + 127) / 128), 128, 0, st>>>(zsrc, fixed, rows, cols, w);
+        DTB_LAUNCH_CHECK("fill_rowscan_kernel");
+        DTB_CUDA(cudaStreamSynchronize(st));
+    } else {
+        const int64_t row_lo = has_above ? -1 : 0, row_hi = has_below ? rows + 1 : rows;
+        DTB_CUDA(cudaMemsetAsync(flags, 0, 8, st));
+        const int kMaxPasses = 200000;
+        for (;;) {
+            DTB_CUDA(cudaMemsetAsync(flags, 0, 4, st));
+            const int burst = passes < 64 ? 4 : 16;  // check the flag every `burst` passes
+            for (int b = 0; b < burst; ++b) {
+                fill_relax_band_kernel<<<(unsigned)ntiles, 256, 0, st>>>(zsrc, fixed, rows, cols, w, tiles_x, flags, row_lo, row_hi,
+                                                                         flags + 1);
+                DTB_LAUNCH_CHECK("fill_relax_band_kernel");
+            }
+            passes += burst;
+            unsigned h[2] = {0, 0};
+            DTB_CUDA(cudaMemcpyAsync(h, flags, 8, cudaMemcpyDeviceToHost, st));
+            DTB_CUDA(cudaStreamSynchronize(st));
+            seam = h[1];
+            if (h[0] == 0) break;
+            if (passes > kMaxPasses) return DTB_ERR_UNSUPPORTED;
+        }
+    }
+    if (passes_host) *passes_host = passes;
+    if (seam_changed_host) *seam_changed_host = seam ? 1 : 0;
     return DTB_OK;
 }

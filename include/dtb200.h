@@ -370,6 +370,24 @@ size_t dtb_fill_workspace_bytes(int64_t rows, int64_t cols);
 int dtb_fill_depressions_f32(float *dem, int64_t rows, int64_t cols, void *ws, size_t ws_bytes,
                              int *iterations_host, void *stream);
 
+/* The same fill over row bands (block-Jacobi: the result equals dtb_fill_depressions_f32 on the
+ * whole raster, bit for bit).  dem_halo is (rows + 2) x cols: row 0 and row rows + 1 are halo rows
+ * holding the neighbour's row next to the seam, read only where has_above / has_below is 1 and
+ * never written; rows 1 .. rows are the band, filled in place.  ws (dtb_fill_band_workspace_bytes)
+ * keeps the band's elevations and seed mask from the INIT call to the SOLVE calls after it.
+ *   mode DTB_FILL_INIT : halo rows = the neighbours' DEM rows (a cell next to nodata across a seam
+ *                        is a seed).  Writes an upper bound of the fill into the band.
+ *   mode DTB_FILL_SOLVE: halo rows = the neighbours' current seam rows of the fill.  Relaxes the
+ *                        band until a pass changes nothing.  *seam_changed_host = 1 if a cell of
+ *                        the band's first or last row was lowered.
+ * The driver runs INIT once, then exchanges the seam rows and runs SOLVE on every band until no
+ * band reports a seam change.  Synchronous.  *passes_host (may be NULL) receives the number of
+ * sweeps (0 for INIT); more than 200000 sweeps in one call return DTB_ERR_UNSUPPORTED. */
+enum { DTB_FILL_INIT = 0, DTB_FILL_SOLVE = 1 };
+size_t dtb_fill_band_workspace_bytes(int64_t rows, int64_t cols);
+int dtb_fill_band_f32(float *dem_halo, int64_t rows, int64_t cols, int has_above, int has_below, int mode,
+                      void *ws, size_t ws_bytes, int *passes_host, int *seam_changed_host, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

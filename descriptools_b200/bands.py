@@ -19,8 +19,10 @@ k logical bands on ONE GPU through the very same kernels and solvers (tests/test
 """
 from __future__ import annotations
 
+import bisect
 import ctypes
 
+import numpy as np
 import torch
 
 TILE = 64
@@ -418,6 +420,241 @@ def fill_rounds(bands, x, max_rounds: int = FILL_MAX_ROUNDS) -> dict:
     raise RuntimeError(f"depression filling over bands did not converge in {max_rounds} rounds")
 
 
+# ---- raster files from bands -------------------------------------------------------------------------
+TIFF_HEADER_BYTES = 16   # the writer reserves them for the header; the chunks follow back to back, each padded to even length
+WRITE_PIECE_BYTES = 64 << 20
+
+
+def device_encoder(lay, raster, c0: int, c1: int):
+    """write_raster's default encoder: chunks [c0, c1) of `raster` (a device tensor holding rows [lay.row_lo, lay.row_hi)
+    of the file) encoded on its device -> (streams back to back, each padded with a zero byte to even length, as a device
+    uint8 tensor; their sizes, np.int64)"""
+    from . import raster as rio
+
+    parts, sizes = [], []
+    cur = torch.cuda.current_stream(raster.device)
+    for _, _, blob, s, _, io in rio.encode_groups(lay, raster, c0, c1):
+        with torch.cuda.stream(io):
+            part = blob.clone()
+        part.record_stream(cur)
+        parts.append(part)
+        sizes.append(s)
+    return torch.cat(parts), np.concatenate(sizes)
+
+
+def _window(lay, lo: int, hi: int):
+    from ._lib import TiffLayout
+
+    w = TiffLayout.from_buffer_copy(lay)
+    w.row_lo, w.row_hi = lo, hi
+    return w
+
+
+def write_plan(edges: list[int], chunk_rows: int, rows: int):
+    """Who encodes what when row bands [edges[i], edges[i+1]) write a file of `chunk_rows`-row chunk-rows.
+    Chunk-row k belongs to the band that holds its first row.  Returns (own, sends):
+      own[i] = (k0, k1, straddle): band i encodes chunk-rows [k0, k1) from its own rows, and chunk-row `straddle` (or None),
+               which runs past its last row, from a staging buffer its successors fill;
+      sends  = [(src band, dst band, first row, end row)]: a band whose first row falls inside a chunk-row sends its rows of
+               that chunk-row to the owner (all of them if the band lies inside the chunk-row)."""
+    own, sends = [], []
+    for i in range(len(edges) - 1):
+        r0, r1 = edges[i], edges[i + 1]
+        k0, k1 = -(-r0 // chunk_rows), -(-r1 // chunk_rows)
+        straddle = k1 - 1 if k0 < k1 and min(k1 * chunk_rows, rows) > r1 else None
+        own.append((k0, k1 if straddle is None else k1 - 1, straddle))
+        if r0 % chunk_rows:
+            k = r0 // chunk_rows
+            sends.append((i, bisect.bisect_right(edges, k * chunk_rows) - 1, r0, min(r1, (k + 1) * chunk_rows)))
+    return own, sends
+
+
+def _write_pieces(w, c0, packed, sizes, offsets, piece_bytes):
+    """chunks c0 .. c0 + len(sizes) - 1 (packed back to back in `packed`, device or host) -> the file at offsets[c0 ...],
+    in pieces of whole chunks of about piece_bytes; a device blob goes through two pinned buffers, the next piece is
+    copied while this one is written"""
+    aligned = (sizes + 1) & ~1
+    rel = np.cumsum(aligned) - aligned
+    pieces, a = [], 0
+    while a < len(sizes):
+        b = max(a + 1, int(np.searchsorted(rel, rel[a] + piece_bytes, side="right")))
+        pieces.append((a, min(b, len(sizes))))
+        a = pieces[-1][1]
+    span = lambda p: (int(rel[p[0]]), int(rel[p[1] - 1] + aligned[p[1] - 1]))
+    if not getattr(packed, "is_cuda", False):
+        host = packed.numpy() if hasattr(packed, "numpy") else packed
+        for p in pieces:
+            lo, hi = span(p)
+            w.write_encoded(c0 + p[0], host[lo:hi], rel[p[0]:p[1]] - lo, sizes[p[0]:p[1]], at=int(offsets[c0 + p[0]]))
+        return
+    cap = max(hi - lo for lo, hi in map(span, pieces))
+    host = [torch.empty(cap, dtype=torch.uint8).pin_memory() for _ in range(min(2, len(pieces)))]
+    copy = torch.cuda.Stream(device=packed.device)
+    copy.wait_stream(torch.cuda.current_stream(packed.device))
+    ready = []
+
+    def fetch(j):
+        lo, hi = span(pieces[j])
+        with torch.cuda.stream(copy):
+            host[j % len(host)][:hi - lo].copy_(packed[lo:hi], non_blocking=True)
+            ev = torch.cuda.Event()
+            ev.record(copy)
+        ready.append(ev)
+
+    fetch(0)
+    for j, p in enumerate(pieces):
+        ready[j].synchronize()
+        if j + 1 < len(pieces):
+            fetch(j + 1)  # into the other buffer: the piece before this one is already written
+        lo, hi = span(p)
+        w.write_encoded(c0 + p[0], host[j % len(host)][:hi - lo], rel[p[0]:p[1]] - lo, sizes[p[0]:p[1]], at=int(offsets[c0 + p[0]]))
+    copy.synchronize()
+
+
+def write_raster(bands, x, path, per_band, meta: dict, encoder=None, piece_bytes: int = WRITE_PIECE_BYTES) -> int:
+    """Write one raster held as row bands into one GeoTIFF, every band encoding and writing its own chunks: no rank
+    ever holds more than its band plus one chunk-row.  The file is byte for byte the one
+    raster.write_from_device(encode="device") writes from the whole raster.
+
+    `bands` are this process's bands (anything with index / grows / cols / dev), `x` the exchange, per_band[k] the
+    contiguous (rows, cols) tensor of local band k, `meta` as for raster.open(path, "w", ...) (width, height and dtype
+    default to the tensors').  `encoder(layout, tensor, c0, c1) -> (packed streams, sizes)` encodes chunks [c0, c1) of a
+    row window (layout.row_lo / row_hi); the default is the device kernel (device_encoder), so only stored or LZW
+    files with predictor 1-3 can be written.
+
+      1. hand-off: a band whose first row falls inside a chunk-row sends its rows of it to the band that owns it
+         (write_plan), which assembles that chunk-row in a staging buffer;
+      2. every band encodes the chunks it owns (they stay where the encoder put them);
+      3. one collective of the per-chunk sizes: every rank computes every chunk's offset (16 header bytes, then the
+         streams in chunk order, each padded to even length);
+      4. the rank holding band 0 created the file (main writer, tags) before that collective; the others open part
+         writers and write their chunks at their offsets, then a collective of the write status; the main writer
+         records the others' chunks and closes (the IFD), and its close status is shared.
+    Any failure on any rank raises on every rank and leaves no file.  Returns the bytes of header and chunks."""
+    from . import raster as rio
+
+    dist_x = isinstance(x, DistExchange)
+    grows, cols, dev = bands[0].grows, bands[0].cols, bands[0].dev
+    meta = dict(meta)
+    meta.setdefault("width", cols)
+    meta.setdefault("height", grows)
+    meta.setdefault("dtype", str(per_band[0].dtype).replace("torch.", ""))
+    if (int(meta["height"]), int(meta["width"])) != (grows, cols):
+        raise rio.RasterError(f"{path}: the bands hold a {grows} x {cols} raster, meta describes {meta['height']} x {meta['width']}")
+    lay, across, n = rio.layout_of(meta)
+    if encoder is None:
+        from ._lib import lib as cuda_lib
+
+        if int(cuda_lib.dtb_tiff_encode_bound(ctypes.byref(lay))) == 0:
+            raise rio.RasterError("row bands write stored or LZW chunks (predictor 1-3) encoded on the device, not this file")
+        encoder = device_encoder
+    ch = lay.chunk_rows
+    edges = band_edges(grows, x.nbands)
+    own, sends = write_plan(edges, ch, grows)
+    local = {b.index: t for b, t in zip(bands, per_band)}
+    for b, t in zip(bands, per_band):
+        if tuple(t.shape) != (edges[b.index + 1] - edges[b.index], cols) or not t.is_contiguous():
+            raise rio.RasterError(f"{path}: band {b.index} must be a contiguous tensor of its {edges[b.index + 1] - edges[b.index]} x {cols} rows")
+
+    # 1. the rows of straddling chunk-rows go to their owners
+    stage = {}
+    for i, (_, _, k) in enumerate(own):
+        if k is not None and i in local:
+            a = k * ch
+            t = local[i]
+            stage[i] = torch.empty((min(a + ch, grows) - a, cols), dtype=t.dtype, device=t.device)
+            stage[i][:edges[i + 1] - a].copy_(t[a - edges[i]:])
+    x.handoff([(src, dst, local[src][a - edges[src]:e - edges[src]] if src in local else None,
+                stage[dst][a - a // ch * ch:e - a // ch * ch] if dst in local else None) for src, dst, a, e in sends])
+
+    # 2. encode what this process owns; 3. the sizes of every chunk
+    main, err, mine = None, None, []
+    try:
+        if 0 in local:
+            main = rio.DatasetWriter(path, **meta)
+        for i in sorted(local):
+            k0, k1, k = own[i]
+            if k1 > k0:
+                mine.append((k0 * across, k1 * across) + tuple(encoder(_window(lay, edges[i], edges[i + 1]), local[i], k0 * across, k1 * across)))
+            if k is not None:
+                a = k * ch
+                mine.append((k * across, (k + 1) * across) + tuple(encoder(_window(lay, a, a + stage[i].shape[0]), stage[i], k * across,
+                                                                           (k + 1) * across)))
+        stage.clear()
+    except Exception as e:  # noqa: BLE001 -- reported to every rank below
+        err = e
+    vec = torch.zeros(n + 1, dtype=torch.int64)
+    vec[0] = 0 if err is None else 1
+    for c0, c1, _, s in mine:
+        vec[1 + c0:1 + c1] = torch.from_numpy(np.asarray(s, dtype=np.int64))
+    vec = _all_sum(x, vec, dev)
+
+    def fail(what, e):
+        if main is not None:
+            main.abort()
+        raise rio.RasterError(f"{path}: {what}" + (f" ({e})" if e is not None else "")) from e
+
+    if vec[0] > 0:
+        fail(f"encoding failed on {int(vec[0])} rank(s)", err)
+    sizes = vec[1:].numpy()
+    if (sizes <= 0).any():
+        fail("a chunk was encoded by no band", None)
+    aligned = (sizes + 1) & ~1
+    offsets = TIFF_HEADER_BYTES + np.cumsum(aligned) - aligned
+    total = int(TIFF_HEADER_BYTES + aligned.sum())
+
+    # 4. every rank writes its chunks at their offsets
+    part = None
+    try:
+        if mine and main is None:
+            part = rio.DatasetWriter(path, part=True, **meta)
+        w = main if main is not None else part
+        if w is not None:
+            got = w.chunk_layout()[0]
+            if any(getattr(got, f) != getattr(lay, f) for f in ("rows", "cols", "bps", "predictor", "compression", "tiled", "chunk_rows", "chunk_cols")):
+                raise rio.RasterError("the writer settled on another chunk layout")
+        for c0, c1, packed, s in mine:
+            _write_pieces(w, c0, packed, np.asarray(s, dtype=np.int64), offsets, piece_bytes)
+        if part is not None:
+            part.close()
+        err = None
+    except Exception as e:  # noqa: BLE001
+        err = e
+        if part is not None:
+            part.abort()
+    bad = int(_all_sum(x, torch.tensor([0 if err is None else 1], dtype=torch.int64), dev)[0])
+    if bad:
+        fail(f"writing failed on {bad} rank(s)", err)
+    # 5. the main writer records the other ranks' chunks and writes the IFD
+    if main is not None:
+        try:
+            written = np.zeros(n, bool)
+            for c0, c1, _, _ in mine:
+                written[c0:c1] = True
+            edge = np.flatnonzero(np.diff(np.concatenate([[1], written.view(np.int8), [1]])))
+            for c0, c1 in zip(edge[::2], edge[1::2]):  # runs of chunks other ranks wrote
+                main.place_chunks(int(c0), offsets[c0:c1], sizes[c0:c1])
+            main.close()
+            err = None
+        except Exception as e:  # noqa: BLE001
+            err = e
+            main.abort()
+    bad = int(_all_sum(x, torch.tensor([0 if main is None or err is None else 1], dtype=torch.int64), dev)[0])
+    if bad:
+        main = None
+        fail("closing the file failed", err)
+    return total
+
+
+def _all_sum(x, t: torch.Tensor, dev) -> torch.Tensor:
+    """sum of a small host int64 tensor over the ranks (nothing to do with all bands in one process)"""
+    if not isinstance(x, DistExchange):
+        return t
+    d = t.to(dev) if torch.device(dev).type == "cuda" else t
+    x.dist.all_reduce(d, group=x.group)
+    return d.cpu()
+
+
 # ---- exchange back-ends ----------------------------------------------------------------------------
 class _GraphedSolver:
     """A boundary solver replayed as a CUDA graph: the solve is ~100 tiny whole-array kernels whose launch
@@ -466,6 +703,11 @@ class LocalExchange:
             if i + 1 < len(items):
                 below.copy_(items[i + 1][0])
 
+    def handoff(self, items):
+        """items = [(src band, dst band, rows to send, where they go)]: row blocks between bands (write_raster)"""
+        for _, _, send, recv in items:
+            recv.copy_(send)
+
     def solve(self, per_band, solver, rounds=ROUNDS):
         out, flag = self.graphed(solver, torch.stack(per_band, 0), rounds)
         self.flags.append(flag.clone())
@@ -492,6 +734,20 @@ class DistExchange:
             ops += [d.P2POp(d.isend, first_row, peer(self.rank - 1), self.group), d.P2POp(d.irecv, above, peer(self.rank - 1), self.group)]
         if self.rank + 1 < self.world:
             ops += [d.P2POp(d.isend, last_row, peer(self.rank + 1), self.group), d.P2POp(d.irecv, below, peer(self.rank + 1), self.group)]
+        if ops:
+            for w in d.batch_isend_irecv(ops):
+                w.wait()
+
+    def handoff(self, items):
+        """items = [(src band, dst band, rows to send or None, where they go or None)]: point-to-point row blocks between
+        bands (write_raster); a rank posts the sends of its band and the receives into its buffers"""
+        d, ops = self.dist, []
+        peer = (lambda r: d.get_global_rank(self.group, r)) if self.group is not None else (lambda r: r)
+        for src, dst, send, recv in items:
+            if src == self.rank:
+                ops.append(d.P2POp(d.isend, send, peer(dst), self.group))
+            if dst == self.rank:
+                ops.append(d.P2POp(d.irecv, recv, peer(src), self.group))
         if ops:
             for w in d.batch_isend_irecv(ops):
                 w.wait()
@@ -553,6 +809,7 @@ class BandRunner:
         mine = range(self.nbands) if isinstance(exchange, LocalExchange) else [exchange.rank]
         self.bands = [Band(i, self.nbands, self.edges[i], self.edges[i + 1], rows, cols, px, river_threshold, n_gfi, b_gfi, device,
                            force_int64) for i in mine]
+        self.geo = {}  # crs / transform of the DEM load_file read: the defaults of write_raster / write_files
 
     def load(self, dem_rows: list[torch.Tensor]):
         """dem_rows[k]: the DEM rows of local band k (device or host tensor)"""
@@ -579,6 +836,7 @@ class BandRunner:
             if src.dtypes[0] != "float32":
                 raise TypeError(f"{path}: row bands take float32 DEMs, the file holds {src.dtypes[0]}")
             nd = src.nodata if nodata is None else nodata
+            self.geo = dict(crs=src.crs, transform=src.transform)
             for b in self.bands:
                 from . import device as _device
 
@@ -767,3 +1025,28 @@ class BandRunner:
 
     def outputs(self) -> list[dict]:
         return [b.outputs() for b in self.bands]
+
+    def write_raster(self, path, per_band: list, **meta) -> int:
+        """One GeoTIFF from a raster held as this process's bands (per_band[k]: local band k's rows, e.g. what downslope()
+        returns), every rank writing its own chunks (write_raster): byte for byte what raster.write_from_device(
+        encode="device") writes from the whole raster.  `meta` as for raster.open(path, "w", ...); crs and transform
+        default to the DEM's from load_file.  Every rank calls it; the file system must be shared by all of them."""
+        meta = {**self.geo, **meta}
+        return write_raster(self.bands, self.x, path, per_band, meta)
+
+    def write_files(self, out_dir, outputs=None, compress: str = "lzw", blocksize: int = 256, **geo) -> dict:
+        """The chain's rasters of the last step() as `out_dir/<name>.tif`, with the metadata pipeline.pipeline_files uses
+        (pipeline.output_meta) and the DEM's georeferencing from load_file (or `geo`): the seven files are byte for byte
+        those pipeline_files writes on one GPU.  Returns {name: path}."""
+        import os
+
+        from .pipeline import STAGE_OUTPUTS, output_meta
+
+        os.makedirs(out_dir, exist_ok=True)
+        paths = {}
+        outs = self.outputs()
+        for name in (STAGE_OUTPUTS if outputs is None else outputs):
+            per_band = [o[name] for o in outs]
+            paths[name] = os.path.join(out_dir, name + ".tif")
+            self.write_raster(paths[name], per_band, **output_meta(name, per_band[0].dtype.is_floating_point, compress, blocksize), **geo)
+        return paths

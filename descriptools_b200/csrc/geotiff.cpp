@@ -576,6 +576,9 @@ struct dtbio_writer {
     std::atomic<uint64_t> pos{0};
     std::vector<uint64_t> offsets, counts;
     std::map<int, Tag> extra;
+    bool part = false;                  // dtbio_open_part: writes chunks only, never the header / IFD
+    bool appended = false;              // chunks went to the end of the file (write_rows / write_encoded)
+    std::map<uint64_t, uint64_t> spans;  // [start, end) of the chunks written or placed at given offsets
 };
 
 namespace {
@@ -718,6 +721,77 @@ int finish(dtbio_writer *w) {
     return DTBIO_OK;
 }
 
+constexpr uint64_t kHeaderBytes = 16;  // reserved for the header, patched in at close (classic TIFF uses 8)
+
+// Chunks first .. first + n - 1 at base + rel[i] (sizes[i] bytes): in the raster, not recorded yet, even, past the
+// header, inside the classic-TIFF 4 GB limit, and disjoint from each other and from every chunk placed before.  On
+// success `r` holds their [start, end) in chunk order.
+int check_placement(const dtbio_writer *w, int64_t first, int64_t n, uint64_t base, const int64_t *rel, const int64_t *sizes,
+                    std::vector<std::pair<uint64_t, uint64_t>> &r) {
+    if (w->appended) return fail(DTBIO_ERR_ORDER, "chunks at given offsets cannot follow chunks appended to the file");
+    if (first + n > w->lay.n_chunks()) return fail(DTBIO_ERR_INVALID, "chunk range outside the raster");
+    r.clear();
+    for (int64_t i = 0; i < n; ++i) {
+        const std::string which = "chunk " + std::to_string(first + i);
+        if (sizes[i] <= 0 || rel[i] < 0) return fail(DTBIO_ERR_INVALID, which + ": bad offset or size");
+        if (w->counts[(size_t)(first + i)]) return fail(DTBIO_ERR_ORDER, which + " written twice");
+        const uint64_t at = base + (uint64_t)rel[i];
+        if (at & 1) return fail(DTBIO_ERR_INVALID, which + ": TIFF offsets must be even");
+        if (at < kHeaderBytes) return fail(DTBIO_ERR_INVALID, which + " overlaps the header");
+        if (!w->big && at + (uint64_t)sizes[i] > 0xFFFFFFF0ull) return fail(DTBIO_ERR_UNSUPPORTED, "classic TIFF would exceed 4 GB: create the file with bigtiff = 1");
+        r.emplace_back(at, at + (uint64_t)sizes[i]);
+    }
+    std::vector<std::pair<uint64_t, uint64_t>> sorted(r);
+    std::sort(sorted.begin(), sorted.end());
+    for (size_t k = 0; k < sorted.size(); ++k) {
+        bool clash = k > 0 && sorted[k].first < sorted[k - 1].second;
+        auto it = w->spans.upper_bound(sorted[k].first);
+        if (it != w->spans.end() && it->first < sorted[k].second) clash = true;
+        if (it != w->spans.begin() && std::prev(it)->second > sorted[k].first) clash = true;
+        if (clash) return fail(DTBIO_ERR_INVALID, "chunks overlap at file offset " + std::to_string(sorted[k].first));
+    }
+    return DTBIO_OK;
+}
+
+void record_placement(dtbio_writer *w, int64_t first, const std::vector<std::pair<uint64_t, uint64_t>> &r) {
+    for (size_t i = 0; i < r.size(); ++i) {
+        w->offsets[(size_t)first + i] = r[i].first;
+        w->counts[(size_t)first + i] = r[i].second - r[i].first;
+        w->spans[r[i].first] = r[i].second;
+    }
+}
+
+// what dtbio_create and dtbio_open_part share: the checks of *info and the layout / BigTIFF decision
+int setup_writer(dtbio_writer *w, const char *path, const dtbio_info *info) {
+    if (info->rows <= 0 || info->cols <= 0) return fail(DTBIO_ERR_INVALID, "raster size must be positive");
+    if (info->dtype < 0 || info->dtype > DTBIO_F64) return fail(DTBIO_ERR_INVALID, "bad dtype");
+    int comp = info->compression == 0 ? DTBIO_COMP_NONE : info->compression;
+    if (comp != DTBIO_COMP_NONE && comp != DTBIO_COMP_LZW && comp != DTBIO_COMP_DEFLATE) return fail(DTBIO_ERR_UNSUPPORTED, "the writer compresses with LZW or Deflate only");
+    int pred = info->predictor == 0 ? 1 : info->predictor;
+    if (pred < 1 || pred > 3) return fail(DTBIO_ERR_INVALID, "bad predictor");
+    if (comp == DTBIO_COMP_NONE) pred = 1;  // a predictor without a codec is not part of the format (GDAL drops it too)
+    if (pred == 3 && info->dtype != DTBIO_F32 && info->dtype != DTBIO_F64) return fail(DTBIO_ERR_INVALID, "predictor 3 needs floating-point samples");
+    if ((info->tile_rows > 0) != (info->tile_cols > 0)) return fail(DTBIO_ERR_INVALID, "give both tile sizes or neither");
+    if (info->tile_rows > 0 && ((info->tile_rows % 16) || (info->tile_cols % 16))) return fail(DTBIO_ERR_INVALID, "tile sizes must be multiples of 16");
+    w->info = *info;
+    w->info.compression = comp;
+    w->info.predictor = pred;
+    const int bps = DT_SIZE[info->dtype];
+    int64_t rps = info->rows_per_strip;
+    if (info->tile_rows == 0 && rps <= 0) rps = std::max<int64_t>(1, 8192 / (info->cols * bps));
+    w->lay.set(info->rows, info->cols, bps, info->tile_rows, info->tile_cols, rps);
+    w->info.rows_per_strip = w->lay.tiled ? 0 : (int32_t)w->lay.ch;
+    const double raw = (double)info->rows * (double)info->cols * bps;
+    w->big = info->bigtiff || raw > (comp == DTBIO_COMP_NONE ? 4.0e9 : 2.0e9);
+    w->info.bigtiff = w->big;
+    w->info.big_endian = 0;
+    w->offsets.assign((size_t)w->lay.n_chunks(), 0);
+    w->counts.assign((size_t)w->lay.n_chunks(), 0);
+    w->path = path;
+    w->pos.store(kHeaderBytes);
+    return DTBIO_OK;
+}
+
 }  // namespace
 
 // =====================================================================================================
@@ -804,36 +878,27 @@ int dtbio_read_rows(dtbio_reader *r, int64_t row0, int64_t nrows, void *dst, int
 int dtbio_create(const char *path, const dtbio_info *info, dtbio_writer **out) {
     if (!path || !info || !out) return fail(DTBIO_ERR_INVALID, "null argument");
     *out = nullptr;
-    if (info->rows <= 0 || info->cols <= 0) return fail(DTBIO_ERR_INVALID, "raster size must be positive");
-    if (info->dtype < 0 || info->dtype > DTBIO_F64) return fail(DTBIO_ERR_INVALID, "bad dtype");
-    int comp = info->compression == 0 ? DTBIO_COMP_NONE : info->compression;
-    if (comp != DTBIO_COMP_NONE && comp != DTBIO_COMP_LZW && comp != DTBIO_COMP_DEFLATE) return fail(DTBIO_ERR_UNSUPPORTED, "the writer compresses with LZW or Deflate only");
-    int pred = info->predictor == 0 ? 1 : info->predictor;
-    if (pred < 1 || pred > 3) return fail(DTBIO_ERR_INVALID, "bad predictor");
-    if (comp == DTBIO_COMP_NONE) pred = 1;  // a predictor without a codec is not part of the format (GDAL drops it too)
-    if (pred == 3 && info->dtype != DTBIO_F32 && info->dtype != DTBIO_F64) return fail(DTBIO_ERR_INVALID, "predictor 3 needs floating-point samples");
-    if ((info->tile_rows > 0) != (info->tile_cols > 0)) return fail(DTBIO_ERR_INVALID, "give both tile sizes or neither");
-    if (info->tile_rows > 0 && ((info->tile_rows % 16) || (info->tile_cols % 16))) return fail(DTBIO_ERR_INVALID, "tile sizes must be multiples of 16");
     return guarded([&]() -> int {
     std::unique_ptr<dtbio_writer> w(new dtbio_writer());
-    w->info = *info;
-    w->info.compression = comp;
-    w->info.predictor = pred;
-    const int bps = DT_SIZE[info->dtype];
-    int64_t rps = info->rows_per_strip;
-    if (info->tile_rows == 0 && rps <= 0) rps = std::max<int64_t>(1, 8192 / (info->cols * bps));
-    w->lay.set(info->rows, info->cols, bps, info->tile_rows, info->tile_cols, rps);
-    w->info.rows_per_strip = w->lay.tiled ? 0 : (int32_t)w->lay.ch;
-    const double raw = (double)info->rows * (double)info->cols * bps;
-    w->big = info->bigtiff || raw > (comp == DTBIO_COMP_NONE ? 4.0e9 : 2.0e9);
-    w->info.bigtiff = w->big;
-    w->info.big_endian = 0;
-    w->offsets.assign((size_t)w->lay.n_chunks(), 0);
-    w->counts.assign((size_t)w->lay.n_chunks(), 0);
-    w->path = path;
+    const int rc = setup_writer(w.get(), path, info);
+    if (rc != DTBIO_OK) return rc;
     w->fd = open(path, O_WRONLY | O_CREAT | O_TRUNC | O_CLOEXEC, 0644);
     if (w->fd < 0) return fail(DTBIO_ERR_IO, std::string("cannot create ") + path + ": " + strerror(errno));
-    w->pos.store(16);  // header is patched in at close
+    *out = w.release();
+    return DTBIO_OK;
+    });
+}
+
+int dtbio_open_part(const char *path, const dtbio_info *info, dtbio_writer **out) {
+    if (!path || !info || !out) return fail(DTBIO_ERR_INVALID, "null argument");
+    *out = nullptr;
+    return guarded([&]() -> int {
+    std::unique_ptr<dtbio_writer> w(new dtbio_writer());
+    const int rc = setup_writer(w.get(), path, info);
+    if (rc != DTBIO_OK) return rc;
+    w->part = true;
+    w->fd = open(path, O_WRONLY | O_CLOEXEC);
+    if (w->fd < 0) return fail(DTBIO_ERR_IO, std::string("cannot open ") + path + ": " + strerror(errno));
     *out = w.release();
     return DTBIO_OK;
     });
@@ -859,12 +924,14 @@ int dtbio_write_rows(dtbio_writer *w, int64_t row0, int64_t nrows, const void *s
     if (row0 < 0 || nrows < 0 || row0 + nrows > L.rows) return fail(DTBIO_ERR_INVALID, "row block outside the raster");
     if (stride < L.cols * L.bps) return fail(DTBIO_ERR_INVALID, "source stride shorter than a row");
     if (nrows == 0) return DTBIO_OK;
+    if (w->part) return fail(DTBIO_ERR_ORDER, "a part writer writes chunks at given offsets only");
     if (row0 % L.ch) return fail(DTBIO_ERR_ORDER, "row block does not start on a chunk boundary");
     if ((row0 + nrows) % L.ch && row0 + nrows != L.rows) return fail(DTBIO_ERR_ORDER, "row block does not end on a chunk boundary");
     int64_t cy0 = row0 / L.ch, cy1 = (row0 + nrows - 1) / L.ch + 1;
     int64_t n = (cy1 - cy0) * L.across;
     for (int64_t i = 0; i < n; ++i)
         if (w->counts[(size_t)(cy0 * L.across + i)]) return fail(DTBIO_ERR_ORDER, "chunk written twice");
+    w->appended = true;
     return guarded([&]() -> int {
         int t = team_size(threads, n);
         std::vector<Scratch> scratch((size_t)t);
@@ -880,10 +947,12 @@ int dtbio_write_encoded(dtbio_writer *w, int64_t first_chunk, int64_t n_chunks, 
     if (n_chunks == 0) return DTBIO_OK;
     if (!blob || !offsets || !sizes) return fail(DTBIO_ERR_INVALID, "null argument");
     if (first_chunk + n_chunks > w->lay.n_chunks()) return fail(DTBIO_ERR_INVALID, "chunk range outside the raster");
+    if (w->part) return fail(DTBIO_ERR_ORDER, "a part writer writes chunks at given offsets only");
     for (int64_t i = 0; i < n_chunks; ++i) {
         if (sizes[i] <= 0 || offsets[i] < 0 || offsets[i] + sizes[i] > blob_bytes) return fail(DTBIO_ERR_INVALID, "chunk " + std::to_string(first_chunk + i) + " lies outside the blob");
         if (w->counts[(size_t)(first_chunk + i)]) return fail(DTBIO_ERR_ORDER, "chunk written twice");
     }
+    w->appended = true;
     uint64_t at = w->pos.fetch_add(((uint64_t)blob_bytes + 1) & ~(uint64_t)1);
     if (!w->big && at + (uint64_t)blob_bytes > 0xFFFFFFF0ull) return fail(DTBIO_ERR_UNSUPPORTED, "classic TIFF would exceed 4 GB: create the file with bigtiff = 1");
     if (!pwrite_all(w->fd, blob, (size_t)blob_bytes, at)) return fail(DTBIO_ERR_IO, std::string("write failed: ") + strerror(errno));
@@ -892,6 +961,47 @@ int dtbio_write_encoded(dtbio_writer *w, int64_t first_chunk, int64_t n_chunks, 
         w->counts[(size_t)(first_chunk + i)] = (uint64_t)sizes[i];
     }
     return DTBIO_OK;
+}
+
+int dtbio_write_encoded_at(dtbio_writer *w, int64_t first_chunk, int64_t n_chunks, const void *blob, int64_t blob_bytes,
+                           const int64_t *offsets, const int64_t *sizes, int64_t file_offset) {
+    if (!w || n_chunks < 0 || first_chunk < 0 || blob_bytes < 0 || file_offset < 0) return fail(DTBIO_ERR_INVALID, "bad argument");
+    if (n_chunks == 0) return DTBIO_OK;
+    if (!blob || !offsets || !sizes) return fail(DTBIO_ERR_INVALID, "null argument");
+    if (file_offset & 1) return fail(DTBIO_ERR_INVALID, "TIFF offsets must be even");
+    if ((uint64_t)file_offset < kHeaderBytes) return fail(DTBIO_ERR_INVALID, "the blob overlaps the header");
+    if (!w->big && (uint64_t)file_offset + (uint64_t)blob_bytes > 0xFFFFFFF0ull) return fail(DTBIO_ERR_UNSUPPORTED, "classic TIFF would exceed 4 GB: create the file with bigtiff = 1");
+    for (int64_t i = 0; i < n_chunks; ++i)
+        if (sizes[i] <= 0 || offsets[i] < 0 || offsets[i] + sizes[i] > blob_bytes) return fail(DTBIO_ERR_INVALID, "chunk " + std::to_string(first_chunk + i) + " lies outside the blob");
+    return guarded([&]() -> int {
+        std::vector<std::pair<uint64_t, uint64_t>> r;
+        const int rc = check_placement(w, first_chunk, n_chunks, (uint64_t)file_offset, offsets, sizes, r);
+        if (rc != DTBIO_OK) return rc;
+        if (!pwrite_all(w->fd, blob, (size_t)blob_bytes, (uint64_t)file_offset)) return fail(DTBIO_ERR_IO, std::string("write failed: ") + strerror(errno));
+        record_placement(w, first_chunk, r);
+        const uint64_t end = (uint64_t)file_offset + (uint64_t)blob_bytes;
+        uint64_t cur = w->pos.load();
+        while (cur < end && !w->pos.compare_exchange_weak(cur, end)) {
+        }
+        return DTBIO_OK;
+    });
+}
+
+int dtbio_place_chunks(dtbio_writer *w, int64_t first_chunk, int64_t n_chunks, const int64_t *file_offsets, const int64_t *sizes) {
+    if (!w || n_chunks < 0 || first_chunk < 0) return fail(DTBIO_ERR_INVALID, "bad argument");
+    if (n_chunks == 0) return DTBIO_OK;
+    if (!file_offsets || !sizes) return fail(DTBIO_ERR_INVALID, "null argument");
+    return guarded([&]() -> int {
+        std::vector<std::pair<uint64_t, uint64_t>> r;
+        const int rc = check_placement(w, first_chunk, n_chunks, 0, file_offsets, sizes, r);
+        if (rc != DTBIO_OK) return rc;
+        record_placement(w, first_chunk, r);
+        uint64_t end = 0, cur = w->pos.load();
+        for (const auto &x : r) end = std::max(end, x.second);
+        while (cur < end && !w->pos.compare_exchange_weak(cur, end)) {
+        }
+        return DTBIO_OK;
+    });
 }
 
 int dtbio_writer_info(const dtbio_writer *w, dtbio_info *info) {
@@ -909,6 +1019,12 @@ int dtbio_close_reader(dtbio_reader *r) {
 
 int dtbio_close_writer(dtbio_writer *w) {
     if (!w) return DTBIO_OK;
+    if (w->part) {  // the main writer owns the header, the IFD and the file's fate
+        int rc = close(w->fd) == 0 ? DTBIO_OK : fail(DTBIO_ERR_IO, std::string("close failed: ") + strerror(errno));
+        w->fd = -1;
+        delete w;
+        return rc;
+    }
     int rc = guarded([&]() -> int { return finish(w); });
     if (close(w->fd) != 0 && rc == DTBIO_OK) rc = fail(DTBIO_ERR_IO, std::string("close failed: ") + strerror(errno));
     w->fd = -1;

@@ -252,13 +252,14 @@ __host__ __device__ inline size_t te_scratch_bytes(const dtb_tiff_layout &L)
 
 // ---- phase 1 (all lanes per row): raster -> scratch chunk.  A partial tile is padded by repeating its last
 // column / row (never read back, compresses well); predictor 3 lays the row out as byte planes, most significant
-// byte of every sample first. ----
+// byte of every sample first.  `raster` holds rows from L.row_lo on (0 for a whole raster); the geometry stays the
+// raster's, so a chunk's stream does not depend on the window it was gathered from. ----
 __host__ __device__ inline void te_gather(const dtb_tiff_layout &L, const ChunkGeom &g, const uint8_t *raster, uint8_t *buf, int lane)
 {
     const int64_t width = g.row_bytes / L.bps;
     for (int64_t r = 0; r < g.stored_rows; ++r) {
         const int64_t rr = r < g.data_rows ? r : g.data_rows - 1;
-        const uint8_t *src = raster + ((g.cy * L.chunk_rows + rr) * L.cols + g.x0) * L.bps;
+        const uint8_t *src = raster + ((g.cy * L.chunk_rows + rr - L.row_lo) * L.cols + g.x0) * L.bps;
         uint8_t *row = buf + r * g.row_bytes;
         for (int64_t i = lane; i < width; i += TD_LANES) {
             const int64_t ii = i < g.ncols ? i : g.ncols - 1;
@@ -400,8 +401,20 @@ int te_validate(const dtb_tiff_layout *L)
     if (v != DTB_OK) return v;
     if (L->compression == TC_DEFLATE || L->compression == TC_PACKBITS) return DTB_ERR_UNSUPPORTED;  // chunks are written stored or LZW-compressed
     if (L->big_endian) return DTB_ERR_UNSUPPORTED;  // files are written little-endian
-    if (L->row_lo != 0 || L->row_hi != 0) return DTB_ERR_UNSUPPORTED;  // whole rasters only
     if (L->predictor == 3 && L->bps < 4) return DTB_ERR_INVALID;
+    return DTB_OK;
+}
+
+// chunks [first, first + n) of an encode call: inside the raster, and with a row window set, inside the window (a
+// chunk-row that ends at the raster's last row counts as ending there, its padding rows are replicated)
+int te_validate_range(const dtb_tiff_layout *L, int64_t first, int64_t n)
+{
+    if (first < 0 || n < 0) return DTB_ERR_INVALID;
+    const int64_t across = td_across(*L);
+    if (first + n > across * ((L->rows + L->chunk_rows - 1) / L->chunk_rows)) return DTB_ERR_INVALID;
+    if (n == 0 || (L->row_lo == 0 && L->row_hi == 0)) return DTB_OK;
+    const int64_t top = first / across * L->chunk_rows, end = ((first + n - 1) / across + 1) * L->chunk_rows;
+    if (top < L->row_lo || (end < L->rows ? end : L->rows) > L->row_hi) return DTB_ERR_INVALID;
     return DTB_OK;
 }
 
@@ -542,9 +555,9 @@ int dtb_tiff_encode_chunks(const dtb_tiff_layout *lay, const void *raster, int64
     const int v = te_validate(lay);
     if (v != DTB_OK) return v;
     if (n_chunks == 0) return DTB_OK;
-    if (!raster || !enc || !sizes || !ws || n_chunks < 0 || first_chunk < 0) return DTB_ERR_INVALID;
-    const int64_t total = td_across(*lay) * ((lay->rows + lay->chunk_rows - 1) / lay->chunk_rows);
-    if (first_chunk + n_chunks > total) return DTB_ERR_INVALID;
+    if (!raster || !enc || !sizes || !ws) return DTB_ERR_INVALID;
+    const int r = te_validate_range(lay, first_chunk, n_chunks);
+    if (r != DTB_OK) return r;
     const size_t per = te_scratch_bytes(*lay);
     if (ws_bytes < per + 256) return DTB_ERR_WORKSPACE;
     int64_t warps = (int64_t)((ws_bytes - 256) / per);
@@ -587,7 +600,9 @@ int dtb_selftest_tiff_encode_host(const dtb_tiff_layout *lay, const void *raster
 {
     const int v = te_validate(lay);
     if (v != DTB_OK) return v;
-    if (!raster_host || !enc_host || !sizes_host || n_chunks < 0) return DTB_ERR_INVALID;
+    if (!raster_host || !enc_host || !sizes_host) return DTB_ERR_INVALID;
+    const int r = te_validate_range(lay, first_chunk, n_chunks);
+    if (r != DTB_OK) return r;
     const dtb_tiff_layout &L = *lay;
     const size_t per = te_scratch_bytes(L), bound = te_bound(L);
     std::vector<uint8_t> scratch(per, 0);

@@ -150,6 +150,13 @@ def output_dtypes(dem_dtype: np.dtype, n_cells: int) -> dict:
     return dict(slope=np.float32, d8=np.uint8, acc=it, fdist=np.float32, idx=it, hand=np.dtype(dem_dtype), gfi=np.float32)
 
 
+def output_meta(name: str, floating: bool, compress: str = "lzw", blocksize: int = 256) -> dict:
+    """file metadata of the chain's raster `name` (pipeline_files, bands.BandRunner.write_files): tiled, the predictor that
+    suits the samples (3 floating point, 2 integers), nodata -100 (0 for the D8 codes, like 12_fdr.tif)"""
+    return dict(compress=compress, predictor=1 if compress in (None, "none") else (3 if floating else 2), tiled=True, blockxsize=blocksize,
+                blockysize=blocksize, nodata=0 if name == "d8" else -100)
+
+
 def pipeline_files(dem_path, out_dir, river_threshold: int, px: float | None = None, n_gfi: float = 0.4,
                    scale_factor: float = 0.1, size: float | None = None, outputs=STAGE_OUTPUTS, compress: str = "lzw",
                    blocksize: int = 256, block_bytes: int = 256 << 20, threads: int = 0, decode: str = "auto", encode: str = "auto",
@@ -196,9 +203,7 @@ def pipeline_files(dem_path, out_dir, river_threshold: int, px: float | None = N
     paths = {}
     for name in outputs:
         t = res[name]
-        kind = "f" if t.dtype.is_floating_point else "i"
         paths[name] = os.path.join(out_dir, name + ".tif")
-        raster.write_from_device(paths[name], t, block_bytes=block_bytes, threads=threads, encode=encode, compress=compress,
-                                 predictor=1 if compress in (None, "none") else (3 if kind == "f" else 2),
-                                 tiled=True, blockxsize=blocksize, blockysize=blocksize, nodata=0 if name == "d8" else -100, **geo)
+        raster.write_from_device(paths[name], t, block_bytes=block_bytes, threads=threads, encode=encode,
+                                 **output_meta(name, t.dtype.is_floating_point, compress, blocksize), **geo)
     return paths

@@ -68,6 +68,9 @@ def _load():
     lib.dtbio_set_tag.argtypes = [c_void_p, c_int, c_int, c_int64, c_void_p]
     lib.dtbio_write_rows.argtypes = [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int]
     lib.dtbio_write_encoded.argtypes = [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p]
+    lib.dtbio_open_part.argtypes = [c_char_p, POINTER(_Info), POINTER(c_void_p)]
+    lib.dtbio_write_encoded_at.argtypes = [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_int64]
+    lib.dtbio_place_chunks.argtypes = [c_void_p, c_int64, c_int64, c_void_p, c_void_p]
     lib.dtbio_bytes_written.restype = c_int64
     lib.dtbio_bytes_written.argtypes = [c_void_p]
     lib.dtbio_close_reader.argtypes = [c_void_p]
@@ -280,13 +283,17 @@ class DatasetReader:
 
 
 class DatasetWriter:
-    """`rio.open(path, "w", **meta)`: `.write(array)` (example.py:216-217) or ordered row blocks."""
+    """`rio.open(path, "w", **meta)`: `.write(array)` (example.py:216-217) or ordered row blocks.
+
+    part=True opens a file another writer created with the same `meta` (a row-band run: every rank writes the chunks it
+    encoded with `write_encoded(..., at=)`); it writes no header, IFD or tags, and closing it leaves the file to the
+    writer that created it."""
 
     mode = "w"
 
     def __init__(self, path, driver="GTiff", width=None, height=None, count=1, dtype=None, crs=None, transform=None, nodata=None,
                  compress=None, predictor=1, tiled=False, blockxsize=256, blockysize=None, bigtiff=False, gdal_metadata=None,
-                 threads: int = 0, **ignored):
+                 threads: int = 0, part: bool = False, **ignored):
         if driver not in ("GTiff", None):
             raise RasterError("only the GTiff driver is written")
         if count != 1:
@@ -311,14 +318,19 @@ class DatasetWriter:
         bt = str(bigtiff).upper()
         info.bigtiff = 1 if bt in ("TRUE", "YES", "1") else 0
         h = c_void_p()
-        _check(lib.dtbio_create(self.name.encode(), byref(info), byref(h)), f"create {self.name}")
-        self._h, self._threads, self.closed = h, threads, False
+        if part:
+            _check(lib.dtbio_open_part(self.name.encode(), byref(info), byref(h)), f"open {self.name} for its chunks")
+        else:
+            _check(lib.dtbio_create(self.name.encode(), byref(info), byref(h)), f"create {self.name}")
+        self._h, self._threads, self.closed, self.part = h, threads, False, part
         _check(lib.dtbio_writer_info(self._h, byref(info)), "dtbio_writer_info")
         self.is_tiled, self.bigtiff = info.tile_rows > 0, bool(info.bigtiff)
         self._compression, self._predictor, self._tile_cols = int(info.compression), int(info.predictor), int(info.tile_cols)
         # row blocks handed to write_rows start and end on multiples of this (or on the last row)
         self.chunk_rows = int(info.tile_rows) if self.is_tiled else int(info.rows_per_strip)
         self.nodata, self.crs, self.transform = nodata, crs, transform
+        if part:
+            return
         try:
             if transform is not None and tuple(transform)[:6] != _IDENTITY:
                 a, b, c, d, e, f = [float(v) for v in tuple(transform)[:6]]
@@ -383,9 +395,10 @@ class DatasetWriter:
         across = -(-self.width // lay.chunk_cols) if self.is_tiled else 1
         return lay, across, across * -(-self.height // lay.chunk_rows)
 
-    def write_encoded(self, first_chunk: int, blob, offsets, sizes):
+    def write_encoded(self, first_chunk: int, blob, offsets, sizes, at: int | None = None):
         """chunks encoded on the device: `blob` (uint8 NumPy array or CPU tensor) holds chunk first_chunk + i at
-        offsets[i] .. offsets[i] + sizes[i]; one file write for the whole group"""
+        offsets[i] .. offsets[i] + sizes[i]; one file write for the whole group.  The blob goes to the end of the file,
+        or with `at=` to that file offset (dtbio_write_encoded_at: even, past the 16 header bytes)."""
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         sizes = np.ascontiguousarray(sizes, dtype=np.int64)
         if hasattr(blob, "data_ptr"):
@@ -393,8 +406,29 @@ class DatasetWriter:
         else:
             blob = np.ascontiguousarray(blob)
             ptr, nbytes = blob.ctypes.data, blob.nbytes
-        _check(lib.dtbio_write_encoded(self._h, first_chunk, sizes.size, c_void_p(ptr), nbytes, c_void_p(offsets.ctypes.data),
-                                       c_void_p(sizes.ctypes.data)), f"write {self.name}")
+        if at is None:
+            _check(lib.dtbio_write_encoded(self._h, first_chunk, sizes.size, c_void_p(ptr), nbytes, c_void_p(offsets.ctypes.data),
+                                           c_void_p(sizes.ctypes.data)), f"write {self.name}")
+        else:
+            _check(lib.dtbio_write_encoded_at(self._h, first_chunk, sizes.size, c_void_p(ptr), nbytes, c_void_p(offsets.ctypes.data),
+                                              c_void_p(sizes.ctypes.data), int(at)), f"write {self.name}")
+
+    def place_chunks(self, first_chunk: int, file_offsets, sizes):
+        """record chunks first_chunk + i that another writer put at file_offsets[i] (sizes[i] bytes) in this file"""
+        file_offsets = np.ascontiguousarray(file_offsets, dtype=np.int64)
+        sizes = np.ascontiguousarray(sizes, dtype=np.int64)
+        if file_offsets.shape != sizes.shape:
+            raise RasterError("place_chunks: one offset per size")
+        _check(lib.dtbio_place_chunks(self._h, first_chunk, sizes.size, c_void_p(file_offsets.ctypes.data), c_void_p(sizes.ctypes.data)),
+               f"place chunks in {self.name}")
+
+    def abort(self):
+        """close without finishing: the file is removed (a part writer only closes its descriptor)"""
+        if not self.closed:
+            self.closed = True
+            lib.dtbio_close_writer(self._h)  # removes the file if a chunk is missing
+        if not self.part and os.path.exists(self.name):
+            os.unlink(self.name)
 
     def write(self, arr, indexes=None):
         a = np.asarray(arr)
@@ -666,29 +700,38 @@ def read_to_device(src, device=None, out=None, block_bytes: int = 256 << 20, thr
             reader.close()
 
 
-def _write_from_device_chunks(w: "DatasetWriter", tensor, block_bytes: int, group_chunks=None) -> None:
-    """write_from_device(encode="device"): groups of whole chunk-rows are encoded by dtb_tiff_encode_chunks (one warp
-    per chunk), packed back to back by dtb_tiff_pack_chunks, copied to a pinned buffer and written with one call
-    (dtbio_write_encoded).  The next group is encoded while this one is copied and written."""
+def encode_groups(lay, tensor, c_lo: int, c_hi: int, block_bytes: int = 256 << 20, group_chunks=None):
+    """Encode chunks [c_lo, c_hi) of the layout `lay` on the tensor's device, in groups of whole chunk-rows: each group
+    is encoded by dtb_tiff_encode_chunks (one warp per chunk) while the group before it is packed by dtb_tiff_pack_chunks.
+    `tensor` is the contiguous raster, or with lay.row_lo / row_hi set the rows [row_lo, row_hi) of it (every chunk must
+    lie inside them).
+
+    Yields (g0, g1, blob, sizes, offsets, stream) per group, in chunk order: `blob` (device uint8) holds the group's
+    streams back to back, stream i at offsets[i] and padded with a zero byte to even length -- the layout of the file --
+    and is ready on `stream`.  It is reused for a later group once the caller asks for the next one, so the caller copies
+    it out on `stream` first."""
     import torch
 
     from ._lib import check
     from ._lib import lib as cuda_lib
 
-    lay, across, n = w.chunk_layout()
     bound = int(cuda_lib.dtb_tiff_encode_bound(ctypes.byref(lay)))
     if bound == 0:
         raise RasterError("encode='device' writes stored or LZW chunks (predictor 1-3, little-endian); use encode='host' for the rest")
     dev = tensor.device
+    across = -(-lay.cols // lay.chunk_cols) if lay.tiled else 1
     chunk_raw = lay.chunk_rows * lay.chunk_cols * lay.bps
+    n = c_hi - c_lo
+    if n <= 0:
+        return
     per_group = group_chunks or _chunks_per_group(n, across, chunk_raw, block_bytes)
-    groups = [(g0, min(n, g0 + per_group)) for g0 in range(0, n, per_group)]
+    groups = [(g0, min(c_hi, g0 + per_group)) for g0 in range(c_lo, c_hi, per_group)]
     nbuf = min(2, len(groups))
     ws_bytes = int(cuda_lib.dtb_tiff_encode_workspace_bytes(ctypes.byref(lay), per_group))
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)  # one workspace: the encode kernels run in order on one stream
     enc = [torch.empty(per_group * bound, dtype=torch.uint8, device=dev) for _ in range(nbuf)]
     sizes_d = [torch.empty(per_group, dtype=torch.int64, device=dev) for _ in range(nbuf)]
-    blob = {"d": None, "h": None}  # packed streams of one group, device and pinned host; grown to what the data needs
+    blob = None  # packed streams of one group; grown to what the data needs
     work, io = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
     work.wait_stream(torch.cuda.current_stream(dev))
     encoded, reusable = [None] * len(groups), [None] * nbuf
@@ -712,23 +755,59 @@ def _write_from_device_chunks(w: "DatasetWriter", tensor, block_bytes: int, grou
         with torch.cuda.stream(io):
             sizes = sizes_d[b][:g1 - g0].cpu().numpy()  # synchronises `io`: the group is encoded
             if (sizes <= 0).any():
-                raise RasterError(f"{w.name}: a chunk did not fit its encode slot")
+                raise RasterError("a chunk did not fit its encode slot")
             aligned = (sizes + 1) & ~1
             offsets = np.cumsum(aligned) - aligned
             total = int(aligned.sum())
             offsets_d = torch.from_numpy(offsets).to(dev)
-            if blob["d"] is None or blob["d"].numel() < total:
-                room = min(per_group * bound, total + total // 4 + 4096)
-                blob["d"] = torch.empty(room, dtype=torch.uint8, device=dev)
-                blob["h"] = torch.empty(room, dtype=torch.uint8).pin_memory()
+            if blob is None or blob.numel() < total:
+                blob = torch.empty(min(per_group * bound, total + total // 4 + 4096), dtype=torch.uint8, device=dev)
+            blob[:total].zero_()  # the pad bytes
             check(cuda_lib.dtb_tiff_pack_chunks(enc[b].data_ptr(), bound, sizes_d[b].data_ptr(), offsets_d.data_ptr(), g1 - g0,
-                                                blob["d"].data_ptr(), io.cuda_stream), "dtb_tiff_pack_chunks")
+                                                blob.data_ptr(), io.cuda_stream), "dtb_tiff_pack_chunks")
             reusable[b] = torch.cuda.Event()
             reusable[b].record(io)
-            blob["h"][:total].copy_(blob["d"][:total], non_blocking=True)
-        io.synchronize()
-        w.write_encoded(g0, blob["h"][:total], offsets, sizes)
+        yield g0, g1, blob[:total], sizes, offsets, io
+    io.synchronize()
     torch.cuda.current_stream(dev).wait_stream(work)
+
+
+def _write_from_device_chunks(w: "DatasetWriter", tensor, block_bytes: int, group_chunks=None) -> None:
+    """write_from_device(encode="device"): encode_groups' packed groups are copied to a pinned buffer and written with
+    one call each (dtbio_write_encoded); the next group is encoded while this one is copied and written."""
+    import torch
+
+    lay, _, n = w.chunk_layout()
+    host = None
+    for g0, _, blob, sizes, offsets, io in encode_groups(lay, tensor, 0, n, block_bytes, group_chunks):
+        if host is None or host.numel() < blob.numel():
+            host = torch.empty(blob.numel() + blob.numel() // 4 + 4096, dtype=torch.uint8).pin_memory()
+        with torch.cuda.stream(io):
+            host[:blob.numel()].copy_(blob, non_blocking=True)
+        io.synchronize()
+        w.write_encoded(g0, host[:blob.numel()], offsets, sizes)
+
+
+def layout_of(meta: dict):
+    """(layout, chunks across, chunks in all) of the file `open(path, "w", **meta)` writes -- for the ranks of a row-band
+    run, which encode their chunks before the file exists.  Strips need an explicit `blockysize`."""
+    from ._lib import TiffLayout
+
+    compress = meta.get("compress")
+    comp = _COMPRESSION[(compress or "none").lower()] if isinstance(compress, (str, type(None))) else int(compress)
+    lay = TiffLayout()
+    lay.rows, lay.cols = int(meta["height"]), int(meta["width"])
+    lay.bps = np.dtype(meta["dtype"]).itemsize
+    lay.compression, lay.big_endian = comp, 0
+    lay.predictor = 1 if comp == 1 else int(meta.get("predictor", 1) or 1)
+    if meta.get("tiled"):
+        lay.tiled, lay.chunk_rows, lay.chunk_cols = 1, int(meta.get("blockysize") or 256), int(meta.get("blockxsize", 256))
+    else:
+        if not meta.get("blockysize"):
+            raise RasterError("give blockysize (rows per strip) for a striped file written by several writers")
+        lay.tiled, lay.chunk_rows, lay.chunk_cols = 0, int(meta["blockysize"]), lay.cols
+    across = -(-lay.cols // lay.chunk_cols) if lay.tiled else 1
+    return lay, across, across * -(-lay.rows // lay.chunk_rows)
 
 
 def write_from_device(path, tensor, block_bytes: int = 256 << 20, threads: int = 0, encode: str = "host",

@@ -329,8 +329,11 @@ typedef struct dtb_tiff_layout {
     int32_t chunk_rows;  /* TileLength or RowsPerStrip                        */
     int32_t chunk_cols;  /* TileWidth (ignored for strips)                    */
     int32_t big_endian;  /* samples stored most significant byte first        */
-    /* decode only: `out` holds raster rows [row_lo, row_hi) (a row band: out points at row row_lo) and only those
-     * rows are stored; both 0 = the whole raster.  Encoding takes whole rasters (both must be 0). */
+    /* a row window, both 0 = the whole raster.  Decoding: `out` holds raster rows [row_lo, row_hi) (a row band: out
+     * points at row row_lo) and only those rows are stored.  Encoding: `raster` points at row row_lo and only rows
+     * [row_lo, row_hi) are read; every chunk encoded must lie inside the window (the last chunk-row may end at `rows`,
+     * its padding rows are replicated as usual), else DTB_ERR_INVALID before any launch.  A chunk's stream is the same
+     * whichever window it was encoded from. */
     int64_t row_lo, row_hi;
 } dtb_tiff_layout;
 size_t dtb_tiff_decode_workspace_bytes(const dtb_tiff_layout *lay, int64_t n_chunks);
@@ -344,11 +347,13 @@ int dtb_selftest_tiff_decode_host(const dtb_tiff_layout *lay, const uint8_t *com
 /* The way back -- replaces the pixel encode inside `rio.open(out, "w", **meta).write(...)` (example.py:216-217):
  * dtb_tiff_encode_chunks: one warp gathers chunk first_chunk + i from the raster (partial tiles padded by edge
  *   replication), applies lay->predictor and encodes it (lay->compression 5 LZW, 1 stored; little-endian only) into
- *   enc + i * dtb_tiff_encode_bound(lay); sizes[i] receives the encoded byte count (DEVICE array).
+ *   enc + i * dtb_tiff_encode_bound(lay); sizes[i] receives the encoded byte count (DEVICE array).  With a row window
+ *   (lay->row_lo / row_hi) `raster` holds only those rows: what one rank of a row-band run holds.
  * dtb_tiff_pack_chunks: copies the n_chunks streams to blob + offsets[i] (DEVICE arrays; the caller computes the
  *   offsets from the sizes), so that one device-to-host copy and one write carry the group
  *   (dtbio_write_encoded, include/dtb200_io.h).
- * dtb_selftest_tiff_encode_host: the encode kernel's per-lane code on the CPU over HOST pointers (CPU test-suite). */
+ * dtb_selftest_tiff_encode_host: the encode kernel's per-lane code on the CPU over HOST pointers, row window included
+ *   (CPU test-suite). */
 size_t dtb_tiff_encode_bound(const dtb_tiff_layout *lay);
 size_t dtb_tiff_encode_workspace_bytes(const dtb_tiff_layout *lay, int64_t n_chunks);
 int dtb_tiff_encode_chunks(const dtb_tiff_layout *lay, const void *raster, int64_t first_chunk, int64_t n_chunks, uint8_t *enc,

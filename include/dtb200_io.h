@@ -103,6 +103,21 @@ int dtbio_write_rows(dtbio_writer *w, int64_t row0, int64_t nrows, const void *s
  * The streams must match the writer's compression / predictor / chunk geometry. */
 int dtbio_write_encoded(dtbio_writer *w, int64_t first_chunk, int64_t n_chunks, const void *blob, int64_t blob_bytes,
                         const int64_t *offsets, const int64_t *sizes);
+/* ---- one file, several writers (a row-band run: every rank writes the chunks it encoded) ----------
+ * The main writer (dtbio_create) owns the file: it writes the header and the IFD at close, and removes the file if a
+ * chunk is missing then.  dtbio_open_part opens the file the main writer created: it checks *info exactly as
+ * dtbio_create does and settles the same layout and BigTIFF decision, but never truncates the file; closing it only
+ * closes its descriptor (no header, no IFD, no unlink).  A part writer takes dtbio_write_encoded_at only.
+ * dtbio_write_encoded_at: as dtbio_write_encoded, but the blob goes to file_offset (even, at least 16: the bytes the
+ *   header reserves) instead of the end of the file; the writer's end of data becomes at least the blob's end.
+ * dtbio_place_chunks: records chunks another writer put at file_offsets[i] (sizes[i] bytes), on the main writer.
+ * Both refuse chunks outside the raster, chunks already recorded, odd offsets or offsets inside the header, chunks
+ * that overlap each other or a chunk placed before, a classic file past 4 GB, and a writer that has appended chunks
+ * (dtbio_write_rows / dtbio_write_encoded): a file takes its chunks either appended or at given offsets. */
+int dtbio_open_part(const char *path, const dtbio_info *info, dtbio_writer **out);
+int dtbio_write_encoded_at(dtbio_writer *w, int64_t first_chunk, int64_t n_chunks, const void *blob, int64_t blob_bytes,
+                           const int64_t *offsets, const int64_t *sizes, int64_t file_offset);
+int dtbio_place_chunks(dtbio_writer *w, int64_t first_chunk, int64_t n_chunks, const int64_t *file_offsets, const int64_t *sizes);
 /* number of bytes in the file so far (header + chunks written) */
 int64_t dtbio_bytes_written(const dtbio_writer *w);
 

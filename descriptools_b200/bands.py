@@ -14,7 +14,7 @@ Here the same decomposition runs in parallel, one process per GPU (torch.distrib
 
 Band seams sit on multiples of 64 rows (the tile edge of the device kernels).  Results are bit-identical to the
 single-GPU run.  The boundary solvers are pure torch (device-agnostic) so the whole driver can be exercised on
-CPU with gloo, with the per-band kernels replaced by a stand-in (tests/test_bands_cpu.py); `LocalBands` runs
+CPU with gloo, with the per-band kernels replaced by a stand-in (tests/test_bands_cpu.py); `LocalExchange` runs
 k logical bands on ONE GPU through the very same kernels and solvers (tests/test_gpu_parity.py).
 """
 from __future__ import annotations
@@ -53,7 +53,17 @@ def band_edges(rows: int, nbands: int) -> list[int]:
 ROUNDS = 6
 
 
-_forest_ws = {}
+_solver_bufs = {}
+
+
+def _solver_buffers(solver: str, dev, out_shape: tuple, ws_bytes: int):
+    """(workspace, int64 output, int32 unresolved flag) of a library solve, allocated on the first call for (solver, device,
+    shape) and reused after: a solve captured in a CUDA graph (_GraphedSolver) replays into the same buffers"""
+    key = (solver, dev.index, out_shape)
+    if key not in _solver_bufs:
+        _solver_bufs[key] = (torch.empty(ws_bytes, dtype=torch.uint8, device=dev), torch.empty(out_shape, dtype=torch.int64, device=dev),
+                             torch.zeros(1, dtype=torch.int32, device=dev))
+    return _solver_bufs[key]
 
 
 def forest_accumulate(nxt: torch.Tensor, base: torch.Tensor, rounds: int = ROUNDS):
@@ -64,12 +74,7 @@ def forest_accumulate(nxt: torch.Tensor, base: torch.Tensor, rounds: int = ROUND
 
         n = nxt.numel()
         nxt, base = nxt.contiguous(), base.contiguous()
-        key = (nxt.device.index, n)
-        if key not in _forest_ws:
-            _forest_ws[key] = (torch.empty(lib.dtb_forest_workspace_bytes(n), dtype=torch.uint8, device=nxt.device),
-                               torch.empty(n, dtype=torch.int64, device=nxt.device),
-                               torch.zeros(1, dtype=torch.int32, device=nxt.device))
-        ws, out, flag = _forest_ws[key]
+        ws, out, flag = _solver_buffers("forest", nxt.device, (n,), lib.dtb_forest_workspace_bytes(n))
         check(lib.dtb_forest_accumulate(nxt.data_ptr(), base.data_ptr(), n, out.data_ptr(), flag.data_ptr(), ws.data_ptr(),
                                         ws.numel(), torch.cuda.current_stream(nxt.device).cuda_stream), "dtb_forest_accumulate")
         return out, flag[0] != 0
@@ -84,8 +89,6 @@ def forest_accumulate(nxt: torch.Tensor, base: torch.Tensor, rounds: int = ROUND
 
 
 _plan_cache = {}
-_hand_ws = {}
-_fa_ws = {}
 
 
 def _plan(n: int, cols: int, dev):
@@ -112,12 +115,7 @@ def solve_flowacc_boundary(summ: torch.Tensor, rounds: int = ROUNDS):
         from ._lib import check, lib
 
         summ = summ.contiguous()
-        key = (summ.device.index, n, cols)
-        if key not in _fa_ws:
-            _fa_ws[key] = (torch.empty(lib.dtb_flowacc_boundary_workspace_bytes(n, cols), dtype=torch.uint8, device=summ.device),
-                           torch.empty((n, 2, cols), dtype=torch.int64, device=summ.device),
-                           torch.zeros(1, dtype=torch.int32, device=summ.device))
-        ws, inflow, flag = _fa_ws[key]
+        ws, inflow, flag = _solver_buffers("flowacc", summ.device, (n, 2, cols), lib.dtb_flowacc_boundary_workspace_bytes(n, cols))
         check(lib.dtb_flowacc_boundary_solve(summ.data_ptr(), n, cols, inflow.data_ptr(), flag.data_ptr(), ws.data_ptr(), ws.numel(),
                                              torch.cuda.current_stream(summ.device).cuda_stream), "dtb_flowacc_boundary_solve")
         return inflow, flag[0] != 0
@@ -148,12 +146,7 @@ def solve_hand_boundary(summ: torch.Tensor, rounds: int = ROUNDS):
         from ._lib import check, lib
 
         summ = summ.contiguous()
-        key = (dev.index, n, cols)
-        if key not in _hand_ws:
-            _hand_ws[key] = (torch.empty(lib.dtb_hand_boundary_workspace_bytes(n, cols), dtype=torch.uint8, device=dev),
-                             torch.empty((n, 8, cols), dtype=torch.int64, device=dev),
-                             torch.zeros(1, dtype=torch.int32, device=dev))
-        ws, res, flag = _hand_ws[key]
+        ws, res, flag = _solver_buffers("hand", dev, (n, 8, cols), lib.dtb_hand_boundary_workspace_bytes(n, cols))
         check(lib.dtb_hand_boundary_solve(summ.data_ptr(), n, cols, int(rounds), res.data_ptr(), flag.data_ptr(), ws.data_ptr(),
                                           ws.numel(), torch.cuda.current_stream(dev).cuda_stream), "dtb_hand_boundary_solve")
         return res, flag[0] != 0
@@ -393,8 +386,8 @@ def fill_rounds(bands, x, max_rounds: int = FILL_MAX_ROUNDS) -> dict:
     halo rows held constant (fill_solve).  A round in which no band lowered a cell of its first or last row leaves every
     band fixed under halos equal to its neighbours' current rows: the whole raster is then the fixed point.
 
-    A band is anything with fill_halo_items / fill_init / fill_solve / fill_release and a `dev` (tests pass NumPy
-    stand-ins).  Returns {"rounds": n, "passes": [relaxation passes of each local band]}."""
+    A band is anything with fill_halo_items / fill_init / fill_solve / fill_release (tests pass NumPy stand-ins).
+    Returns {"rounds": n, "passes": [relaxation passes of each local band]}."""
     items = [b.fill_halo_items() for b in bands]
     x.halo(items)  # the DEM rows next to the seams: a cell beside nodata across a seam is a seed
     passes = [0] * len(bands)
@@ -408,11 +401,7 @@ def fill_rounds(bands, x, max_rounds: int = FILL_MAX_ROUNDS) -> dict:
                 p, s = b.fill_solve()
                 passes[k] += p
                 moved += s
-            if isinstance(x, DistExchange):
-                t = torch.tensor([moved], dtype=torch.int64, device=bands[0].dev)
-                x.dist.all_reduce(t, group=x.group)
-                moved = int(t.item())
-            if moved == 0:
+            if int(x.all_sum(torch.tensor([moved], dtype=torch.int64))[0]) == 0:
                 return {"rounds": rnd, "passes": passes}
     finally:
         for b in bands:
@@ -516,7 +505,7 @@ def write_raster(bands, x, path, per_band, meta: dict, encoder=None, piece_bytes
     ever holds more than its band plus one chunk-row.  The file is byte for byte the one
     raster.write_from_device(encode="device") writes from the whole raster.
 
-    `bands` are this process's bands (anything with index / grows / cols / dev), `x` the exchange, per_band[k] the
+    `bands` are this process's bands (anything with index / grows / cols), `x` the exchange, per_band[k] the
     contiguous (rows, cols) tensor of local band k, `meta` as for raster.open(path, "w", ...) (width, height and dtype
     default to the tensors').  `encoder(layout, tensor, c0, c1) -> (packed streams, sizes)` encodes chunks [c0, c1) of a
     row window (layout.row_lo / row_hi); the default is the device kernel (device_encoder), so only stored or LZW
@@ -533,8 +522,7 @@ def write_raster(bands, x, path, per_band, meta: dict, encoder=None, piece_bytes
     Any failure on any rank raises on every rank and leaves no file.  Returns the bytes of header and chunks."""
     from . import raster as rio
 
-    dist_x = isinstance(x, DistExchange)
-    grows, cols, dev = bands[0].grows, bands[0].cols, bands[0].dev
+    grows, cols = bands[0].grows, bands[0].cols
     meta = dict(meta)
     meta.setdefault("width", cols)
     meta.setdefault("height", grows)
@@ -587,7 +575,7 @@ def write_raster(bands, x, path, per_band, meta: dict, encoder=None, piece_bytes
     vec[0] = 0 if err is None else 1
     for c0, c1, _, s in mine:
         vec[1 + c0:1 + c1] = torch.from_numpy(np.asarray(s, dtype=np.int64))
-    vec = _all_sum(x, vec, dev)
+    vec = x.all_sum(vec)
 
     def fail(what, e):
         if main is not None:
@@ -622,7 +610,7 @@ def write_raster(bands, x, path, per_band, meta: dict, encoder=None, piece_bytes
         err = e
         if part is not None:
             part.abort()
-    bad = int(_all_sum(x, torch.tensor([0 if err is None else 1], dtype=torch.int64), dev)[0])
+    bad = int(x.all_sum(torch.tensor([0 if err is None else 1], dtype=torch.int64))[0])
     if bad:
         fail(f"writing failed on {bad} rank(s)", err)
     # 5. the main writer records the other ranks' chunks and writes the IFD
@@ -639,26 +627,18 @@ def write_raster(bands, x, path, per_band, meta: dict, encoder=None, piece_bytes
         except Exception as e:  # noqa: BLE001
             err = e
             main.abort()
-    bad = int(_all_sum(x, torch.tensor([0 if main is None or err is None else 1], dtype=torch.int64), dev)[0])
+    bad = int(x.all_sum(torch.tensor([0 if main is None or err is None else 1], dtype=torch.int64))[0])
     if bad:
         main = None
         fail("closing the file failed", err)
     return total
 
 
-def _all_sum(x, t: torch.Tensor, dev) -> torch.Tensor:
-    """sum of a small host int64 tensor over the ranks (nothing to do with all bands in one process)"""
-    if not isinstance(x, DistExchange):
-        return t
-    d = t.to(dev) if torch.device(dev).type == "cuda" else t
-    x.dist.all_reduce(d, group=x.group)
-    return d.cpu()
-
-
 # ---- exchange back-ends ----------------------------------------------------------------------------
 class _GraphedSolver:
-    """A boundary solver replayed as a CUDA graph: the solve is ~100 tiny whole-array kernels whose launch
-    overhead (not their run time) is what rank 0 would otherwise spend between the two collectives."""
+    """A boundary solver replayed as a CUDA graph: on CUDA tensors a solve is one library call of about ten kernel
+    launches and memsets, whose launch overhead (not their run time) every rank would otherwise spend between the two
+    collectives."""
 
     def __init__(self):
         self.cache = {}
@@ -687,13 +667,30 @@ class _GraphedSolver:
         return out, flag
 
 
-class LocalExchange:
+class _Exchange:
+    """Where the bands live, as the band driver sees it: `nbands`, the indices of the bands this process holds
+    (`local_bands`), row exchanges between bands (halo, handoff), small collectives (all_sum, broadcast) and the
+    boundary solves.  `flags` collects the unresolved flag of every solve until the driver checks them."""
+
+    def __init__(self, nbands: int, local_bands):
+        self.nbands, self.local_bands = nbands, local_bands
+        self.flags = []
+        self.graphed = _GraphedSolver()
+
+    def solve(self, per_band, solver, rounds=ROUNDS):
+        """per_band: the summaries of this process's bands.  Every band's summary is gathered here and this process solves
+        the (small) boundary graph itself, keeping its own bands' answers: one collective per solve, and no rank waits
+        for rank 0 to prepare and scatter."""
+        res, flag = self.graphed(solver, self._gather(per_band), rounds)
+        self.flags.append(flag.clone())
+        return [res[i].clone() for i in self.local_bands]
+
+
+class LocalExchange(_Exchange):
     """All bands live in this process (tests; k logical bands on one GPU)."""
 
     def __init__(self, nbands):
-        self.nbands = nbands
-        self.flags = []
-        self.graphed = _GraphedSolver()
+        super().__init__(nbands, range(nbands))
 
     def halo(self, items):
         """items[i] = (first_row, last_row, halo_above_dst, halo_below_dst) of band i"""
@@ -708,13 +705,18 @@ class LocalExchange:
         for _, _, send, recv in items:
             recv.copy_(send)
 
-    def solve(self, per_band, solver, rounds=ROUNDS):
-        out, flag = self.graphed(solver, torch.stack(per_band, 0), rounds)
-        self.flags.append(flag.clone())
-        return [out[i].clone() for i in range(len(per_band))]
+    def all_sum(self, t: torch.Tensor) -> torch.Tensor:
+        """one process: the sum is t"""
+        return t
+
+    def broadcast(self, t: torch.Tensor, band: int):
+        """one process: t already holds band `band`'s rows"""
+
+    def _gather(self, per_band):
+        return torch.stack(per_band, 0)
 
 
-class DistExchange:
+class DistExchange(_Exchange):
     """One band per rank over torch.distributed (NCCL on GPUs, gloo in the CPU tests)."""
 
     def __init__(self, group=None):
@@ -722,39 +724,48 @@ class DistExchange:
 
         self.dist, self.group = dist, group
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
-        self.nbands = self.world
-        self.flags = []
-        self.graphed = _GraphedSolver()
+        super().__init__(self.world, [self.rank])
+        # NCCL reduces device tensors only: all_sum takes a host tensor through this GPU
+        self.dev = torch.device("cuda", torch.cuda.current_device()) if dist.get_backend(group) == "nccl" else None
+
+    def _peer(self, r: int) -> int:
+        """the global rank of rank r of the group: what P2POp and broadcast take"""
+        return r if self.group is None else self.dist.get_global_rank(self.group, r)
 
     def halo(self, items):
+        """items = [(first_row, last_row, halo_above_dst, halo_below_dst)] of this rank's band"""
         (first_row, last_row, above, below), = items
-        d, ops = self.dist, []
-        peer = (lambda r: d.get_global_rank(self.group, r)) if self.group is not None else (lambda r: r)  # P2POp wants global ranks
-        if self.rank > 0:
-            ops += [d.P2POp(d.isend, first_row, peer(self.rank - 1), self.group), d.P2POp(d.irecv, above, peer(self.rank - 1), self.group)]
-        if self.rank + 1 < self.world:
-            ops += [d.P2POp(d.isend, last_row, peer(self.rank + 1), self.group), d.P2POp(d.irecv, below, peer(self.rank + 1), self.group)]
-        if ops:
-            for w in d.batch_isend_irecv(ops):
-                w.wait()
+        r, blocks = self.rank, []
+        if r > 0:
+            blocks += [(r, r - 1, first_row, None), (r - 1, r, None, above)]
+        if r + 1 < self.world:
+            blocks += [(r, r + 1, last_row, None), (r + 1, r, None, below)]
+        self.handoff(blocks)
 
     def handoff(self, items):
         """items = [(src band, dst band, rows to send or None, where they go or None)]: point-to-point row blocks between
-        bands (write_raster); a rank posts the sends of its band and the receives into its buffers"""
+        bands; a rank posts the sends of its band and the receives into its buffers, in the order of `items`"""
         d, ops = self.dist, []
-        peer = (lambda r: d.get_global_rank(self.group, r)) if self.group is not None else (lambda r: r)
         for src, dst, send, recv in items:
             if src == self.rank:
-                ops.append(d.P2POp(d.isend, send, peer(dst), self.group))
+                ops.append(d.P2POp(d.isend, send, self._peer(dst), self.group))
             if dst == self.rank:
-                ops.append(d.P2POp(d.irecv, recv, peer(src), self.group))
+                ops.append(d.P2POp(d.irecv, recv, self._peer(src), self.group))
         if ops:
             for w in d.batch_isend_irecv(ops):
                 w.wait()
 
-    def solve(self, per_band, solver, rounds=ROUNDS):
-        """all-gather the summaries; every rank solves the (small) boundary graph itself and keeps its own answer: one
-        collective per solve and no rank waits for rank 0 to prepare and scatter"""
+    def all_sum(self, t: torch.Tensor) -> torch.Tensor:
+        """t summed over the ranks, on t's device"""
+        d = t if self.dev is None else t.to(self.dev)
+        self.dist.all_reduce(d, group=self.group)
+        return d.to(t.device)
+
+    def broadcast(self, t: torch.Tensor, band: int):
+        """t on every rank := t on the rank holding band `band`"""
+        self.dist.broadcast(t, src=self._peer(band), group=self.group)
+
+    def _gather(self, per_band):
         (mine,), d = per_band, self.dist
         mine = mine.contiguous()
         everyone = torch.empty((self.world,) + tuple(mine.shape), dtype=mine.dtype, device=mine.device)
@@ -762,9 +773,7 @@ class DistExchange:
             d.all_gather_into_tensor(everyone.view(-1), mine.view(-1), group=self.group)
         else:  # gloo (the CPU tests)
             d.all_gather(list(everyone.unbind(0)), mine, group=self.group)
-        res, flag = self.graphed(solver, everyone, rounds)
-        self.flags.append(flag.clone())
-        return [res[self.rank].clone()]
+        return everyone
 
 
 def bind_to_gpu_numa(device_index: int) -> list[int] | None:
@@ -806,9 +815,8 @@ class BandRunner:
         self.edges = band_edges(rows, self.nbands)
         if device is None:
             device = torch.device("cuda", torch.cuda.current_device())
-        mine = range(self.nbands) if isinstance(exchange, LocalExchange) else [exchange.rank]
         self.bands = [Band(i, self.nbands, self.edges[i], self.edges[i + 1], rows, cols, px, river_threshold, n_gfi, b_gfi, device,
-                           force_int64) for i in mine]
+                           force_int64) for i in exchange.local_bands]
         self.geo = {}  # crs / transform of the DEM load_file read: the defaults of write_raster / write_files
 
     def load(self, dem_rows: list[torch.Tensor]):
@@ -915,8 +923,10 @@ class BandRunner:
         B = self.bands
         rec(0)
         items = [(b.dem_buf[2:4], b.dem_buf[b.rows:b.rows + 2], b.dem_buf[0:2], b.dem_buf[b.rows + 2:b.rows + 4]) for b in B]
-        if isinstance(self.x, DistExchange) and B[0].dem_buf.is_cuda and min(b.rows for b in B) > 4:
-            # the exchange runs on its own stream while the stencil does every row that needs no halo
+        if B[0].dem_buf.is_cuda and min(b.rows for b in B) > 4:
+            # the exchange runs on its own stream while the stencil does every row that needs no halo.  It writes only
+            # halo rows, which those rows do not read, and reads only DEM rows (its neighbours' ones, for local bands),
+            # which the stencil does not write
             main = torch.cuda.current_stream(B[0].dev)
             if not hasattr(self, "_comm"):
                 self._comm = torch.cuda.Stream(device=B[0].dev)
@@ -961,7 +971,6 @@ class BandRunner:
         from ._lib import check, lib
 
         dev = self.bands[0].dev
-        dist_x = isinstance(self.x, DistExchange)
         h = max(int(halo_rows), 1)
         while True:
             items, wins = [], []
@@ -988,9 +997,7 @@ class BandRunner:
                 outs.append(out)
                 complete &= (b.first or ha == self.edges[b.index] - self.edges[b.index - 1]) and \
                             (b.last or hb == self.edges[b.index + 2] - self.edges[b.index + 1])
-            state = torch.stack([esc[0], torch.tensor(0 if complete else 1, dtype=torch.int64, device=dev)])
-            if dist_x:
-                self.x.dist.all_reduce(state, group=self.x.group)
+            state = self.x.all_sum(torch.stack([esc[0], torch.tensor(0 if complete else 1, dtype=torch.int64, device=dev)]))
             escaped, widenable = (int(v) for v in state.tolist())
             if escaped == 0:
                 return outs
@@ -1012,9 +1019,8 @@ class BandRunner:
             if i in mine:
                 full_dem[a:e].copy_(mine[i].dem)
                 full_d8[a:e].copy_(mine[i].d8)
-            if isinstance(self.x, DistExchange):
-                self.x.dist.broadcast(full_dem[a:e], src=i, group=self.x.group)
-                self.x.dist.broadcast(full_d8[a:e], src=i, group=self.x.group)
+            self.x.broadcast(full_dem[a:e], i)
+            self.x.broadcast(full_d8[a:e], i)
         outs = []
         for b in self.bands:
             out = torch.empty((b.rows, self.cols), dtype=torch.float32, device=dev)

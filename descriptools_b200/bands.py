@@ -422,7 +422,7 @@ def device_encoder(lay, raster, c0: int, c1: int):
 
     parts, sizes = [], []
     cur = torch.cuda.current_stream(raster.device)
-    for _, _, blob, s, _, io in rio.encode_groups(lay, raster, c0, c1):
+    for _, _, blob, s, io in rio.encode_groups(lay, raster, c0, c1):
         with torch.cuda.stream(io):
             part = blob.clone()
         part.record_stream(cur)
@@ -456,48 +456,6 @@ def write_plan(edges: list[int], chunk_rows: int, rows: int):
             k = r0 // chunk_rows
             sends.append((i, bisect.bisect_right(edges, k * chunk_rows) - 1, r0, min(r1, (k + 1) * chunk_rows)))
     return own, sends
-
-
-def _write_pieces(w, c0, packed, sizes, offsets, piece_bytes):
-    """chunks c0 .. c0 + len(sizes) - 1 (packed back to back in `packed`, device or host) -> the file at offsets[c0 ...],
-    in pieces of whole chunks of about piece_bytes; a device blob goes through two pinned buffers, the next piece is
-    copied while this one is written"""
-    aligned = (sizes + 1) & ~1
-    rel = np.cumsum(aligned) - aligned
-    pieces, a = [], 0
-    while a < len(sizes):
-        b = max(a + 1, int(np.searchsorted(rel, rel[a] + piece_bytes, side="right")))
-        pieces.append((a, min(b, len(sizes))))
-        a = pieces[-1][1]
-    span = lambda p: (int(rel[p[0]]), int(rel[p[1] - 1] + aligned[p[1] - 1]))
-    if not getattr(packed, "is_cuda", False):
-        host = packed.numpy() if hasattr(packed, "numpy") else packed
-        for p in pieces:
-            lo, hi = span(p)
-            w.write_encoded(c0 + p[0], host[lo:hi], rel[p[0]:p[1]] - lo, sizes[p[0]:p[1]], at=int(offsets[c0 + p[0]]))
-        return
-    cap = max(hi - lo for lo, hi in map(span, pieces))
-    host = [torch.empty(cap, dtype=torch.uint8).pin_memory() for _ in range(min(2, len(pieces)))]
-    copy = torch.cuda.Stream(device=packed.device)
-    copy.wait_stream(torch.cuda.current_stream(packed.device))
-    ready = []
-
-    def fetch(j):
-        lo, hi = span(pieces[j])
-        with torch.cuda.stream(copy):
-            host[j % len(host)][:hi - lo].copy_(packed[lo:hi], non_blocking=True)
-            ev = torch.cuda.Event()
-            ev.record(copy)
-        ready.append(ev)
-
-    fetch(0)
-    for j, p in enumerate(pieces):
-        ready[j].synchronize()
-        if j + 1 < len(pieces):
-            fetch(j + 1)  # into the other buffer: the piece before this one is already written
-        lo, hi = span(p)
-        w.write_encoded(c0 + p[0], host[j % len(host)][:hi - lo], rel[p[0]:p[1]] - lo, sizes[p[0]:p[1]], at=int(offsets[c0 + p[0]]))
-    copy.synchronize()
 
 
 def write_raster(bands, x, path, per_band, meta: dict, encoder=None, piece_bytes: int = WRITE_PIECE_BYTES) -> int:
@@ -602,7 +560,7 @@ def write_raster(bands, x, path, per_band, meta: dict, encoder=None, piece_bytes
             if any(getattr(got, f) != getattr(lay, f) for f in ("rows", "cols", "bps", "predictor", "compression", "tiled", "chunk_rows", "chunk_cols")):
                 raise rio.RasterError("the writer settled on another chunk layout")
         for c0, c1, packed, s in mine:
-            _write_pieces(w, c0, packed, np.asarray(s, dtype=np.int64), offsets, piece_bytes)
+            rio.write_packed(w, c0, packed, s, piece_bytes, offsets=offsets[c0:c1])
         if part is not None:
             part.close()
         err = None

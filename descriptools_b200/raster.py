@@ -454,12 +454,13 @@ class DatasetWriter:
         return self
 
     def __exit__(self, exc_type, *exc):
-        if exc_type is not None:
+        if exc_type is None:
+            self.close()
+        elif not self.closed:
             # leave no half-written file behind; the library unlinks it when chunks are missing
             self.closed = True
             lib.dtbio_close_writer(self._h)
-            return False
-        self.close()
+        return False
 
     def __del__(self):
         if not getattr(self, "closed", True):
@@ -486,6 +487,48 @@ def _block_rows(src_rows: int, chunk_rows: int, cols: int, itemsize: int, target
     want = max(1, target_bytes // max(1, cols * itemsize))
     chunk_rows = max(1, chunk_rows)
     return min(max(chunk_rows, want // chunk_rows * chunk_rows), max(src_rows, 1))
+
+
+def _rows(buf, k: int, br: int, rows: int, cols: int, dtype):
+    """block k of `rows` rows streamed `br` at a time: (its first row, its rows as an (n, cols) `dtype` view of `buf`)"""
+    n = min(br, rows - k * br)
+    return k * br, buf[:n * cols * dtype.itemsize].view(dtype).view(n, cols)
+
+
+def _to_device(count: int, cap: int, fill, send, copy) -> None:
+    """Host -> device through min(2, count) pinned uint8 buffers of `cap` bytes: fill(k, buf) writes piece k on the host
+    while piece k-1 is sent, then send(k, buf) enqueues on `copy` what reads the buffer.  Returns when all has run."""
+    import torch
+
+    stage = [torch.empty(cap, dtype=torch.uint8, pin_memory=True) for _ in range(min(2, count))]
+    copy.wait_stream(torch.cuda.current_stream(copy.device))  # the destination may reuse memory the current stream still works on
+    for k in range(count):
+        fill(k, stage[k % len(stage)])
+        copy.synchronize()  # piece k-1 is sent: its buffer takes piece k+1
+        with torch.cuda.stream(copy):
+            send(k, stage[k % len(stage)])
+    copy.synchronize()
+
+
+def _from_device(count: int, cap: int, fetch, drain, copy, ready) -> None:
+    """Device -> host through min(2, count) pinned uint8 buffers of `cap` bytes: fetch(k, buf) enqueues the copy of piece
+    k on `copy` (after the work on `ready`), drain(k, buf) consumes it on the host while piece k+1 is copied."""
+    import torch
+
+    stage = [torch.empty(cap, dtype=torch.uint8, pin_memory=True) for _ in range(min(2, count))]
+
+    def enqueue(k):
+        with torch.cuda.stream(copy):
+            fetch(k, stage[k % len(stage)])
+
+    copy.wait_stream(ready)
+    if count:
+        enqueue(0)
+    for k in range(count):
+        copy.synchronize()  # piece k has landed: nothing is enqueued behind it
+        if k + 1 < count:
+            enqueue(k + 1)  # into the other buffer, drained already
+        drain(k, stage[k % len(stage)])
 
 
 _WARPS_IN_FLIGHT = 148 * 8 * 4  # the codec kernels keep one chunk per resident warp (csrc/tiffcodec.cu)
@@ -563,7 +606,7 @@ def _check_chunk_table(name: str, off: np.ndarray, cnt: np.ndarray, file_size: i
 
 def _read_to_device_chunks(reader, out, block_bytes: int, copy, group_chunks=None, rows=None):
     """read_to_device(decode="device"): the compressed chunks go over PCIe as they lie in the file and are decoded
-    by dtb_tiff_decode_chunks, one warp per chunk.  File spans are read into two pinned staging buffers; reading
+    by dtb_tiff_decode_chunks, one warp per chunk.  File spans are staged through pinned memory (_to_device); reading
     span k+1 overlaps the copy and decode of span k on `copy`."""
     import torch
 
@@ -591,41 +634,37 @@ def _read_to_device_chunks(reader, out, block_bytes: int, copy, group_chunks=Non
         hi = int((off[g0:g1] + cnt[g0:g1])[live].max()) if live.any() else 0
         spans.append((lo, hi))
     biggest = max(1, max(hi - lo for lo, hi in spans))
-    stage = [torch.empty(biggest, dtype=torch.uint8).pin_memory() for _ in range(min(2, len(groups)))]
-    comp = [torch.empty(biggest, dtype=torch.uint8, device=dev) for _ in stage]
+    comp = [torch.empty(biggest, dtype=torch.uint8, device=dev) for _ in range(min(2, len(groups)))]  # reused in order on `copy`
     ws_bytes = int(cuda_lib.dtb_tiff_decode_workspace_bytes(ctypes.byref(lay), per_group))
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
     status = torch.zeros(1, dtype=torch.int64, device=dev)
-    copy.wait_stream(torch.cuda.current_stream(dev))
-    free = [None] * len(stage)
+
+    def fill(k, buf):
+        lo, hi = spans[k]
+        view = memoryview(buf.numpy())[:hi - lo]
+        got = 0
+        while got < hi - lo:
+            m = os.preadv(fd, [view[got:]], lo + got)
+            if m <= 0:
+                raise RasterError(f"{reader.name}: file ends inside a chunk")
+            got += m
+
+    def send(k, buf):
+        (g0, g1), (lo, hi), c = groups[k], spans[k], comp[k % len(comp)]
+        rel = off[g0:g1] - np.uint64(lo)
+        rel[cnt[g0:g1] == 0] = 0
+        table = torch.from_numpy(np.concatenate([rel, cnt[g0:g1]]).view(np.int64))
+        c[:hi - lo].copy_(buf[:hi - lo], non_blocking=True)
+        table_d = table.to(dev)  # small and pageable: synchronous with respect to the host, ordered on `copy`
+        check(cuda_lib.dtb_tiff_decode_chunks(ctypes.byref(lay), c.data_ptr(), table_d.data_ptr(), table_d.data_ptr() + 8 * (g1 - g0),
+                                              g0, g1 - g0, out.data_ptr(), ws.data_ptr(), ws_bytes, status.data_ptr(), copy.cuda_stream),
+              "dtb_tiff_decode_chunks")
+
     fd = os.open(reader.name, os.O_RDONLY)
     try:
-        for k, ((g0, g1), (lo, hi)) in enumerate(zip(groups, spans)):
-            s = k % len(stage)
-            if free[s] is not None:
-                free[s].synchronize()  # the copy out of this staging buffer (and the decode behind it) has finished
-            view = memoryview(stage[s].numpy())[:hi - lo]
-            got = 0
-            while got < hi - lo:
-                m = os.preadv(fd, [view[got:]], lo + got)
-                if m <= 0:
-                    raise RasterError(f"{reader.name}: file ends inside a chunk")
-                got += m
-            rel = off[g0:g1] - np.uint64(lo)
-            rel[cnt[g0:g1] == 0] = 0
-            table = torch.from_numpy(np.concatenate([rel, cnt[g0:g1]]).view(np.int64))
-            with torch.cuda.stream(copy):
-                comp[s][:hi - lo].copy_(stage[s][:hi - lo], non_blocking=True)
-                table_d = table.to(dev)  # small and pageable: synchronous with respect to the host, ordered on `copy`
-                check(cuda_lib.dtb_tiff_decode_chunks(ctypes.byref(lay), comp[s].data_ptr(), table_d.data_ptr(),
-                                                      table_d.data_ptr() + 8 * (g1 - g0), g0, g1 - g0, out.data_ptr(),
-                                                      ws.data_ptr(), ws_bytes, status.data_ptr(), copy.cuda_stream),
-                      "dtb_tiff_decode_chunks")
-                free[s] = torch.cuda.Event()
-                free[s].record(copy)
+        _to_device(len(groups), biggest, fill, send, copy)
     finally:
         os.close(fd)
-    copy.synchronize()
     code = int(status.item())
     if code:
         reason = {1: "corrupt compressed stream", 2: "pre-6.0 LZW", 3: "chunk decodes short"}.get(code & 7, "decode error")
@@ -676,24 +715,18 @@ def read_to_device(src, device=None, out=None, block_bytes: int = 256 << 20, thr
         elif tuple(out.shape) != shape or out.dtype != tdt or not out.is_cuda:
             raise RasterError("read_to_device: `out` must be a CUDA tensor of the (band of the) raster's shape and dtype")
         br = _block_rows(nrows, reader.block_shapes[0][0], cols, out.element_size(), block_bytes)
-        stage = [torch.empty((br, cols), dtype=tdt).pin_memory() for _ in range(2 if nrows > br else 1)]
-        free = [None] * len(stage)
+
+        def fill(k, buf):
+            r0, rows_k = _rows(buf, k, br, nrows, cols, tdt)
+            reader.read_rows(first + r0, rows_k.shape[0], rows_k, threads)
+
+        def send(k, buf):
+            r0, rows_k = _rows(buf, k, br, nrows, cols, tdt)
+            out[r0:r0 + rows_k.shape[0]].copy_(rows_k, non_blocking=True)
+
         copy = stream if stream is not None else torch.cuda.Stream(device=out.device)
-        copy.wait_stream(torch.cuda.current_stream(out.device))  # `out` may reuse memory the current stream still works on
-        for k, r0 in enumerate(range(0, nrows, br)):
-            n = min(br, nrows - r0)
-            s = k % len(stage)
-            if free[s] is not None:
-                free[s].synchronize()  # the copy that last read this staging block has finished
-            reader.read_rows(first + r0, n, stage[s], threads)
-            with torch.cuda.stream(copy):
-                out[r0:r0 + n].copy_(stage[s][:n], non_blocking=True)
-                free[s] = torch.cuda.Event()
-                free[s].record(copy)
+        _to_device(-(-nrows // br), br * cols * out.element_size(), fill, send, copy)
         torch.cuda.current_stream(out.device).wait_stream(copy)
-        for ev in free:
-            if ev is not None:
-                ev.synchronize()  # the staging blocks die with this frame
         return out
     finally:
         if reader is not src:
@@ -706,10 +739,10 @@ def encode_groups(lay, tensor, c_lo: int, c_hi: int, block_bytes: int = 256 << 2
     `tensor` is the contiguous raster, or with lay.row_lo / row_hi set the rows [row_lo, row_hi) of it (every chunk must
     lie inside them).
 
-    Yields (g0, g1, blob, sizes, offsets, stream) per group, in chunk order: `blob` (device uint8) holds the group's
-    streams back to back, stream i at offsets[i] and padded with a zero byte to even length -- the layout of the file --
-    and is ready on `stream`.  It is reused for a later group once the caller asks for the next one, so the caller copies
-    it out on `stream` first."""
+    Yields (g0, g1, blob, sizes, stream) per group, in chunk order: `blob` (device uint8) holds the group's streams back
+    to back, each padded with a zero byte to even length -- the layout of the file, what write_packed takes -- and is
+    ready on `stream`.  It is reused for a later group once the caller asks for the next one, so the caller copies it out
+    first."""
     import torch
 
     from ._lib import check
@@ -767,25 +800,44 @@ def encode_groups(lay, tensor, c_lo: int, c_hi: int, block_bytes: int = 256 << 2
                                                 blob.data_ptr(), io.cuda_stream), "dtb_tiff_pack_chunks")
             reusable[b] = torch.cuda.Event()
             reusable[b].record(io)
-        yield g0, g1, blob[:total], sizes, offsets, io
+        yield g0, g1, blob[:total], sizes, io
     io.synchronize()
     torch.cuda.current_stream(dev).wait_stream(work)
 
 
-def _write_from_device_chunks(w: "DatasetWriter", tensor, block_bytes: int, group_chunks=None) -> None:
-    """write_from_device(encode="device"): encode_groups' packed groups are copied to a pinned buffer and written with
-    one call each (dtbio_write_encoded); the next group is encoded while this one is copied and written."""
+def write_packed(w: "DatasetWriter", first_chunk: int, packed, sizes, piece_bytes: int, offsets=None, ready=None) -> None:
+    """Write chunks first_chunk + i (sizes[i] bytes each), packed back to back in `packed` as encode_groups packs them, in
+    chunk order and in pieces of whole chunks of about `piece_bytes`: appended (the same bytes as one append of the whole
+    blob), or with `offsets` at file offset offsets[i] (a row band's chunks).  A device blob is staged through pinned
+    memory after the work on `ready` (default: the current stream), the next piece copied while this one is written; a
+    host blob (NumPy array or CPU tensor) is written as it lies."""
     import torch
 
-    lay, _, n = w.chunk_layout()
-    host = None
-    for g0, _, blob, sizes, offsets, io in encode_groups(lay, tensor, 0, n, block_bytes, group_chunks):
-        if host is None or host.numel() < blob.numel():
-            host = torch.empty(blob.numel() + blob.numel() // 4 + 4096, dtype=torch.uint8).pin_memory()
-        with torch.cuda.stream(io):
-            host[:blob.numel()].copy_(blob, non_blocking=True)
-        io.synchronize()
-        w.write_encoded(g0, host[:blob.numel()], offsets, sizes)
+    sizes = np.asarray(sizes, dtype=np.int64)
+    aligned = (sizes + 1) & ~1
+    rel = np.cumsum(aligned) - aligned
+    pieces, a = [], 0  # (first, end) chunk of each piece, its bytes [lo, hi) in `packed`
+    while a < len(sizes):
+        b = min(len(sizes), max(a + 1, int(np.searchsorted(rel, rel[a] + piece_bytes, side="right"))))
+        pieces.append((a, b, int(rel[a]), int(rel[b - 1] + aligned[b - 1])))
+        a = b
+
+    def put(j, buf):  # piece j, which starts at buf[0]
+        a, b, lo, hi = pieces[j]
+        w.write_encoded(first_chunk + a, buf[:hi - lo], rel[a:b] - lo, sizes[a:b], at=None if offsets is None else int(offsets[a]))
+
+    if not getattr(packed, "is_cuda", False):
+        host = packed.numpy() if hasattr(packed, "numpy") else packed
+        for j, p in enumerate(pieces):
+            put(j, host[p[2]:])
+        return
+
+    def fetch(j, buf):
+        _, _, lo, hi = pieces[j]
+        buf[:hi - lo].copy_(packed[lo:hi], non_blocking=True)
+
+    _from_device(len(pieces), max(hi - lo for _, _, lo, hi in pieces), fetch, put, torch.cuda.Stream(device=packed.device),
+                 ready if ready is not None else torch.cuda.current_stream(packed.device))
 
 
 def layout_of(meta: dict):
@@ -816,9 +868,10 @@ def write_from_device(path, tensor, block_bytes: int = 256 << 20, threads: int =
     (width / height / dtype default to the tensor's).  Returns the number of bytes written.
 
     encode="host": row blocks; block k+1 is copied to its pinned staging buffer while the thread team encodes block k.
-    encode="device": the chunks are encoded on the device and only the compressed bytes cross PCIe (stored and LZW
-    files; anything else raises -- nothing falls back silently).
-    encode="auto": "device" when device_encode_supported(writer), else "host"."""
+    encode="device": the chunks are encoded on the device and only the compressed bytes cross PCIe, in pieces of about
+    `block_bytes` (write_packed) (stored and LZW files; anything else raises -- nothing falls back silently).
+    encode="auto": "device" when device_encode_supported(writer), else "host".
+    A failed call leaves no file."""
     import torch
 
     if encode not in ("host", "device", "auto"):
@@ -839,39 +892,24 @@ def write_from_device(path, tensor, block_bytes: int = 256 << 20, threads: int =
         if encode == "device":
             if not tensor.is_contiguous():
                 raise RasterError("write_from_device(encode='device') needs a contiguous tensor")
-            _write_from_device_chunks(w, tensor, block_bytes, group_chunks)
-            total = w.bytes_written
-            w.close()
-            return total
-        br = _block_rows(rows, w.chunk_rows, cols, tensor.element_size(), block_bytes)
-        stage = [torch.empty((br, cols), dtype=tensor.dtype).pin_memory() for _ in range(2 if rows > br else 1)]
-        copy = torch.cuda.Stream(device=tensor.device)
-        copy.wait_stream(torch.cuda.current_stream(tensor.device))
-        starts = list(range(0, rows, br))
-        done = []
+            lay, _, n = w.chunk_layout()
+            for g0, _, blob, sizes, io in encode_groups(lay, tensor, 0, n, block_bytes, group_chunks):
+                write_packed(w, g0, blob, sizes, block_bytes, ready=io)
+        else:
+            br = _block_rows(rows, w.chunk_rows, cols, tensor.element_size(), block_bytes)
 
-        def fetch(k):
-            r0 = starts[k]
-            n = min(br, rows - r0)
-            with torch.cuda.stream(copy):
-                stage[k % len(stage)][:n].copy_(tensor[r0:r0 + n], non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(copy)
-            done.append(ev)
+            def fetch(k, buf):
+                r0, rows_k = _rows(buf, k, br, rows, cols, tensor.dtype)
+                rows_k.copy_(tensor[r0:r0 + rows_k.shape[0]], non_blocking=True)
 
-        fetch(0)
-        for k, r0 in enumerate(starts):
-            n = min(br, rows - r0)
-            done[k].synchronize()
-            if k + 1 < len(starts) and len(stage) > 1:
-                fetch(k + 1)  # lands in the other staging block while this one is encoded
-            w.write_rows(r0, stage[k % len(stage)][:n])
-            if k + 1 < len(starts) and len(stage) == 1:
-                fetch(k + 1)
+            def drain(k, buf):
+                w.write_rows(*_rows(buf, k, br, rows, cols, tensor.dtype))
+
+            _from_device(-(-rows // br), br * cols * tensor.element_size(), fetch, drain, torch.cuda.Stream(device=tensor.device),
+                         torch.cuda.current_stream(tensor.device))
         total = w.bytes_written
         w.close()
         return total
     except Exception:
-        w.closed = True
-        lib.dtbio_close_writer(w._h)
+        w.abort()
         raise

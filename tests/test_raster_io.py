@@ -246,6 +246,32 @@ def test_errors_are_reported_not_guessed(tmp_path):
     assert not os.path.exists(tmp_path / "y.tif")
 
 
+def _count_closes(monkeypatch):
+    """dtbio_close_writer wrapped: counts the calls per handle and forwards only the first (a second one would free the
+    handle twice)"""
+    calls, real = {}, rio.lib.dtbio_close_writer
+
+    def close_once(h):
+        calls[h.value] = calls.get(h.value, 0) + 1
+        return real(h) if calls[h.value] == 1 else 0
+
+    monkeypatch.setattr(rio.lib, "dtbio_close_writer", close_once)
+    return calls
+
+
+def test_writer_closed_inside_its_with_block_is_closed_once(tmp_path, monkeypatch):
+    calls = _count_closes(monkeypatch)
+    a = _rand((64, 80), "float32", seed=1)
+    p = tmp_path / "c.tif"
+    with pytest.raises(RuntimeError, match="after close"):
+        with rio.open(p, "w", width=80, height=64, dtype="float32", compress="lzw", tiled=True, blockxsize=32, blockysize=32) as w:
+            w.write(a)
+            w.close()
+            raise RuntimeError("after close")
+    assert list(calls.values()) == [1]
+    np.testing.assert_array_equal(rio.open(p).read(1), a)  # complete, so it stays
+
+
 def _decode_like_the_device(path, first=0, count=None, rows=None):
     """the tile-decoding kernel's per-lane code (csrc/tiffcodec.cu), run lane by lane on the CPU by the library's self-test
     entry point: same geometry, LZW, byte order, predictor and store code the warps execute"""
@@ -810,6 +836,51 @@ def test_tiles_encoded_on_the_device(tmp_path, dtype, layout, compress, predicto
     np.testing.assert_array_equal(rio.open(p).read(1), a)
     with pytest.raises(rio.RasterError, match="encode='host'"):
         rio.write_from_device(p, t, encode="device", compress="deflate")
+    assert not os.path.exists(p)
+
+
+@pytest.mark.gpu
+def test_device_encoded_groups_are_written_in_pieces(tmp_path, monkeypatch):
+    """a small block_bytes cuts every group into pieces of whole chunks (both pinned buffers reused): the file is byte
+    for byte the one a single append per group gives"""
+    import torch
+
+    a = _rand((1000, 777), "float32", seed=15)
+    t = torch.from_numpy(a).cuda()
+    kw = dict(encode="device", compress="lzw", predictor=3, tiled=True, blockxsize=128, blockysize=128)
+    one, many = tmp_path / "one.tif", tmp_path / "many.tif"
+    rio.write_from_device(one, t, **kw)  # one group, one piece
+    writes, real = [], rio.DatasetWriter.write_encoded
+
+    def counted(self, first_chunk, *args, **kwargs):
+        writes.append(first_chunk)
+        return real(self, first_chunk, *args, **kwargs)
+
+    monkeypatch.setattr(rio.DatasetWriter, "write_encoded", counted)
+    rio.write_from_device(many, t, block_bytes=100_000, **kw)  # two groups of 28 chunks, pieces of about 100 kB
+    assert len(writes) > 4 and writes == sorted(writes)
+    assert one.read_bytes() == many.read_bytes()
+    np.testing.assert_array_equal(rio.open(many).read(1), a)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("encode", ["host", "device"])
+def test_failed_write_from_device_closes_once_and_leaves_no_file(tmp_path, monkeypatch, encode):
+    import torch
+
+    calls = _count_closes(monkeypatch)
+    real_close = rio.DatasetWriter.close
+
+    def close_then_fail(self):
+        real_close(self)
+        raise rio.RasterError("injected close failure")
+
+    monkeypatch.setattr(rio.DatasetWriter, "close", close_then_fail)
+    t = torch.from_numpy(_rand((300, 200), "float32", seed=2)).cuda()
+    p = tmp_path / "f.tif"
+    with pytest.raises(rio.RasterError, match="injected"):
+        rio.write_from_device(p, t, encode=encode, compress="lzw", tiled=True, blockxsize=64, blockysize=64)
+    assert list(calls.values()) == [1]
     assert not os.path.exists(p)
 
 

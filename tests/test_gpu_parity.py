@@ -44,17 +44,36 @@ def synth(rows, cols, seed, holes=True):
 
 
 # ---- slope + D8 -------------------------------------------------------------------------------
+def misaligned(t):
+    """the same values in a contiguous view that starts 4 bytes into its buffer: not 16-byte aligned"""
+    buf = torch.empty(t.numel() + 1, dtype=t.dtype, device=t.device)
+    v = buf[1:].view(t.shape)
+    v.copy_(t)
+    assert v.data_ptr() % 16 != 0
+    return v
+
+
 def check_slope_d8(mods, dem, px):
-    """all three launch forms (slope only, D8 only, both outputs -- the fused kernel of the chain) against the oracle"""
+    """all three launch forms (slope only, D8 only, both outputs -- the fused kernel of the chain) against the oracle;
+    then all three again on a DEM that is not 16-byte aligned, which only the generic kernel takes"""
     from descriptools_b200 import device
 
     with np.errstate(all="ignore"):
         s_ref, d_ref = oracle.slope_d8(dem, px)
     np.testing.assert_array_equal(mods["slope"].sloper(dem, px).astype(np.float32), s_ref)
     np.testing.assert_array_equal(mods["flowhand"].flow_direction_d8(dem, px), d_ref)
-    s, d = device.slope_d8(torch.from_numpy(np.ascontiguousarray(dem)).cuda(), px)
+    t = torch.from_numpy(np.ascontiguousarray(dem)).cuda()
+    s, d = device.slope_d8(t, px)
     np.testing.assert_array_equal(s.cpu().numpy(), s_ref)
     np.testing.assert_array_equal(d.cpu().numpy(), d_ref)
+    g = misaligned(t)
+    s, d = device.slope_d8(g, px)
+    np.testing.assert_array_equal(s.cpu().numpy(), s_ref, err_msg="generic kernel, both outputs")
+    np.testing.assert_array_equal(d.cpu().numpy(), d_ref, err_msg="generic kernel, both outputs")
+    s, _ = device.slope_d8(g, px, want_d8=False)
+    np.testing.assert_array_equal(s.cpu().numpy(), s_ref, err_msg="generic kernel, slope only")
+    _, d = device.slope_d8(g, px, want_slope=False)
+    np.testing.assert_array_equal(d.cpu().numpy(), d_ref, err_msg="generic kernel, D8 only")
 
 
 @pytest.mark.parametrize("shape", [(1, 1), (1, 7), (5, 1), (3, 3), (64, 128), (65, 129), (130, 260), (257, 516), (100, 1534 // 2)])
@@ -100,10 +119,12 @@ def test_slope_d8_near_tie_card_vs_diag(mods, px):
 
 @pytest.mark.parametrize("px", [12.5, 25.0, 0.5, 30.0, 1.0, 7.77])
 def test_slope_d8_tma_path_exact(mods, px):
-    """the TMA kernel's lean strip (width % 4 == 0): power-of-two and general 100/px, several tiles, pits everywhere."""
+    """the lean strip on both kernels: power-of-two and general 100/px, several tiles, pits everywhere; crops to widths
+    4k + 1, 4k + 2 and 4k + 3 (generic kernel only) end every row in a ragged group of fewer than four cells."""
     rng = np.random.default_rng(int(px * 100))
     dem = (np.cumsum(rng.standard_normal((300, 512)), axis=1) * 3 + rng.standard_normal((300, 512)) + 400).astype(np.float32)
-    check_slope_d8(mods, dem, px)
+    for cols in (512, 509, 510, 511):
+        check_slope_d8(mods, np.ascontiguousarray(dem[:, :cols]), px)
 
 
 @pytest.mark.parametrize("scale", [1e-30, 1e-38, 1e-42, 1e25, 1e36])

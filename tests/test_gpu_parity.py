@@ -8,7 +8,7 @@ import pytest
 import torch
 
 import oracle
-from helpers import example_inputs, load, sha
+from helpers import example_inputs, hand_fused_vs_oracle, listed_tiles, load, serpentine_d8, sha, synth
 
 pytestmark = pytest.mark.gpu
 
@@ -30,17 +30,6 @@ def mods():
 @pytest.fixture(scope="module")
 def ex():
     return example_inputs()
-
-
-def synth(rows, cols, seed, holes=True):
-    dem = oracle.synth_dem(rows, cols, 0, seed)
-    if holes:
-        rng = np.random.default_rng(seed)
-        for _ in range(6):
-            r, c = int(rng.integers(2, rows - 12)), int(rng.integers(2, cols - 12))
-            dem[r:r + int(rng.integers(1, 10)), c:c + int(rng.integers(1, 10))] = -100
-        dem[rows // 2, :5] = -100
-    return oracle.priority_flood_eps(dem)
 
 
 # ---- slope + D8 -------------------------------------------------------------------------------
@@ -972,50 +961,23 @@ def test_downslope_window_marks_escaping_walks():
     np.testing.assert_array_equal(out[~flagged].cpu().numpy(), ref[a:b][~flagged].cpu().numpy())
 
 
-def _hand_fused_vs_oracle(d8, dem, thr):
-    from descriptools_b200 import _lib, device
-
-    acc_ref, _ = oracle.flow_accumulation(d8)
-    river = (acc_ref > thr).astype(np.int8)
-    f_ref, i_ref, h_ref = oracle.flow_hand_index(dem, d8, river, PX)
-    g_ref = oracle.gfi(h_ref, acc_ref, i_ref, 0.4, 0.1, PX)
-    t8, td = torch.from_numpy(d8).cuda(), torch.from_numpy(dem).cuda()
-    _lib.profile_enable(True)
-    try:
-        acc = device.flow_accumulation(t8, fuse_hand_threshold=thr)
-        out = device.hand(t8, td, PX, acc=acc, river_threshold=thr, gfi_params=(0.4, 0.1, PX), entry_done=True)
-        torch.cuda.synchronize()
-        prof = _lib.profile_collect()
-    finally:
-        _lib.profile_enable(False)
-    np.testing.assert_array_equal(acc.cpu().numpy(), acc_ref)
-    np.testing.assert_array_equal(out["idx"].cpu().numpy(), i_ref)
-    np.testing.assert_array_equal(out["hand"].cpu().numpy(), h_ref)
-    np.testing.assert_allclose(out["fdist"].cpu().numpy(), f_ref, rtol=RTOL, atol=0)
-    np.testing.assert_allclose(out["gfi"].cpu().numpy(), g_ref, rtol=RTOL, atol=ATOL)
-    return prof
-
-
 def test_fused_hand_tiles_beyond_the_compact_counters():
-    """in-tile paths of 256+ moves of one kind (a serpentine: 4000+ cardinal moves per tile; a staircase of
-    diagonal / cardinal pairs) do not fit the 8-bit counters of the compact tile pass: those tiles must go through
-    the list to the 64-bit pass and still match the oracle"""
-    rows, cols = 200, 300
-    d8 = np.zeros((rows, cols), np.uint8)
-    for r in range(rows):
-        east = r % 2 == 0
-        d8[r, :] = 1 if east else 16
-        d8[r, cols - 1 if east else 0] = 4
-    dem = (np.arange(rows * cols, dtype=np.float32)[::-1].reshape(rows, cols) * 0.01 + 5).copy()
-    prof = _hand_fused_vs_oracle(d8, dem, rows * cols - 500)
-    assert prof["hand_tile_kernel<listed>"][0] > 0.0
-    # 260 x 260 block of a diagonal staircase: SE moves in 64-cell tiles stay below 64 per tile; stretch them with a
-    # zigzag E, SE, E, SE ... limited to one tile row so that one tile sees > 255 moves in total but < 256 of each kind
+    """in-tile paths of 256+ moves of one kind do not fit the 8-bit counters of the compact tile pass: a serpentine
+    narrower than a tile (3 800+ cardinal moves inside one tile) must go through the list to the 64-bit pass and
+    still match the oracle.  Serpentines and rows wider than a tile leave every tile within 64 + 64 moves: the
+    compact pass keeps them."""
+    for rows, cols, listed in ((200, 300, False), (200, 60, True)):
+        d8 = serpentine_d8(rows, cols)
+        dem = (np.arange(rows * cols, dtype=np.float32)[::-1].reshape(rows, cols) * 0.01 + 5).copy()
+        prof = hand_fused_vs_oracle(d8, dem, rows * cols - 500)
+        assert prof["hand_tile_kernel<listed>"][0] > 0.0
+        assert (listed_tiles(rows, cols) > 0) == listed, (rows, cols)
+    # every row flows east across ten tiles
     d8 = np.full((128, 640), 1, np.uint8)
     d8[:, -1] = 4
     d8[-1, -1] = 4
     dem = np.linspace(900, 1, 128 * 640, dtype=np.float32).reshape(128, 640).copy()
-    _hand_fused_vs_oracle(d8, dem, 128 * 640 - 700)
+    hand_fused_vs_oracle(d8, dem, 128 * 640 - 700)
 
 
 def test_fused_hand_random_codes_with_cycles():
@@ -1026,7 +988,8 @@ def test_fused_hand_random_codes_with_cycles():
                     p=[.03, .2, .1, .2, .1, .1, .08, .08, .08, .015, .015])
     dem = (rng.standard_normal(d8.shape) * 10 + 100).astype(np.float32)
     dem[rng.random(d8.shape) < 0.02] = -100
-    _hand_fused_vs_oracle(d8, dem, 3)
+    hand_fused_vs_oracle(d8, dem, 3)
+    assert listed_tiles(150, 200) > 0
 
 
 def test_hand_boundary_solver_cuda_equals_torch():

@@ -26,9 +26,11 @@
 //       and GFI from the gathered accumulation of the river cell, written once.
 // Distance = n_card*px + n_diag*(px*sqrt(2)) in f64 (the reference adds the same terms one
 // move at a time, flowhand.py:803-824; the two agree far below f32 resolution).
-// GFI = ln(b) + n*ln(A_r*size^2) - ln(H + 0.01) in f64: the reference's
-// log(b*pow(A_r*size^2, n)/(H+0.01)) (gfi.py:292-294) rearranged to drop the pow; both are
-// correctly rounded far below the f32 the result is stored in.
+// GFI = ln(b) + n*ln(A_r*size^2) - ln(H + 0.01) in f64 with the short logarithms of common.cuh: the
+// reference's log(b*pow(A_r*size^2, n)/(H+0.01)) (gfi.py:292-294) rearranged to drop the pow.  The two
+// agree to (|n| + 2) * 3e-9 plus the f32 rounding of the stored result where |n| <= 8 and 1e-30 < b < 1e30
+// (the domain pointwise.cu's log form serves), including n = 0 with A_r = 0 and NaN / infinite HAND values.
+// Outside that domain the rearranged form stays finite where the reference's pow overflows.
 #include <math.h>
 #include <stdlib.h>
 
@@ -167,11 +169,16 @@ template <> struct HandOps<float> {
     static __device__ __forceinline__ bool is_nd(float z) { return z == ND_F; }
     static __device__ __forceinline__ float sub(float a, float b) { return a - b; }
     static __device__ __forceinline__ float nd() { return ND_F; }
+    // fast_log_pos needs a finite argument (it reads +inf as 1024 ln 2): for a NaN / +inf HAND (a non-finite DEM cell)
+    // subtracting H gives the reference's NaN / -inf (NaN where ln b + n ln(A_r size^2) is +inf too).  Two f32
+    // instructions per cell; correcting the f64 log instead cost the issue-bound tile pass ~3 % (B200, 40k x 40k).
+    static __device__ __forceinline__ void fix_nonfinite(float &g, float h) { if (!(fabsf(h) < INFINITY)) g -= h; }
 };
 template <> struct HandOps<int16_t> {
     static __device__ __forceinline__ bool is_nd(int16_t z) { return z == ND_I; }
     static __device__ __forceinline__ int16_t sub(int16_t a, int16_t b) { return (int16_t)(a - b); }  // numpy i16 wrap
     static __device__ __forceinline__ int16_t nd() { return (int16_t)ND_I; }
+    static __device__ __forceinline__ void fix_nonfinite(float &, int16_t) {}
 };
 
 // flowhand.py:436-438
@@ -278,7 +285,8 @@ __device__ __forceinline__ void resolve_exit(const TileView &v, int64_t r0, int6
             exit_z[slot] = (o.hand || o.gfi) ? dem[loc] : (TD)0;
             if (o.gfi) racc = (double)acc[loc];  // river_accumulation, gfi.py:141-143
         }
-        exit_l1[slot] = o.gfi ? o.gfi_logb + o.gfi_n * fast_log(racc * o.gfi_s2) : 0.0;
+        // n = 0: ln b for every A_r, as pow(A_r size^2, 0) = 1 is in the reference (n * ln 0 would be NaN); same at the two sites below
+        exit_l1[slot] = o.gfi ? (o.gfi_n == 0.0 ? o.gfi_logb : o.gfi_logb + o.gfi_n * fast_log(racc * o.gfi_s2)) : 0.0;
     }
 }
 
@@ -320,7 +328,10 @@ __device__ __forceinline__ void finish_cell(const HandOut &o, const bool want_h,
     if (want_h && ok && !HandOps<TD>::is_nd(z)) {  // flowhand.py:436-438
         h = HandOps<TD>::sub(z, zr);
         if (h < (TD)0 && h != HandOps<TD>::nd()) h = (TD)0;
-        if (want_g && !(h <= HandOps<TD>::nd())) g = (float)(l1 - fast_log_pos((double)h + 0.01));  // gfi.py:289-294
+        if (want_g && !(h <= HandOps<TD>::nd())) {  // gfi.py:289-294
+            g = (float)(l1 - fast_log_pos((double)h + 0.01));
+            HandOps<TD>::fix_nonfinite(g, h);
+        }
     }
     hd = h;
     gf = g;
@@ -481,7 +492,7 @@ __device__ __forceinline__ void hand_tile_body(const int tile, const TileView &v
             } else if (kind == KIND_RIVER) {  // river cell inside this tile: s2.x = its local index in the band
                 idx = (int64_t)s2.x + o.idx_offset;
                 if (o.hand || o.gfi) zr = dem[s2.x];
-                if (o.gfi) l1 = o.gfi_logb + o.gfi_n * fast_log((double)acc[s2.x] * o.gfi_s2);  // gfi.py:141-143
+                if (o.gfi) l1 = (o.gfi_n == 0.0 ? o.gfi_logb : o.gfi_logb + o.gfi_n * fast_log((double)acc[s2.x] * o.gfi_s2));  // gfi.py:141-143
             }
             finish_cell<TD, IDX>(o, o.hand || o.gfi, o.gfi != nullptr, kind, nd, nc, idx, zr, l1, z[i], fd[i], ix[i], hd[i], gf[i]);
         }
@@ -659,7 +670,7 @@ hand_tile_compact_kernel(TileView v, const TD *__restrict__ dem, const ACC *__re
                 const int64_t loc = (r0 + (int64_t)(rp >> 6)) * v.cols + c0 + (int64_t)(rp & 63u);
                 idx = loc + o.idx_offset;
                 if (w_hd || w_gf) zr = dem[loc];
-                if (w_gf) l1 = o.gfi_logb + o.gfi_n * fast_log((double)acc[loc] * o.gfi_s2);  // gfi.py:141-143
+                if (w_gf) l1 = (o.gfi_n == 0.0 ? o.gfi_logb : o.gfi_logb + o.gfi_n * fast_log((double)acc[loc] * o.gfi_s2));  // gfi.py:141-143
             }
             finish_cell<TD, IDX>(o, w_hd || w_gf, w_gf, kind, nd, nc, idx, zr, l1, z[i], fd[i], ix[i], hd[i], gf[i]);
         }

@@ -65,21 +65,36 @@ def listed_tiles(rows, cols):
     return int(ws[128:132].view(torch.int32).item())
 
 
-def hand_fused_vs_oracle(d8, dem, thr, px=PX):
-    """fused flow accumulation + HAND (entry_done) on a D8 grid against the oracle; returns the kernel profile"""
+def misaligned(t):
+    """the same values in a contiguous view that starts one element (2, 4 or 8 bytes) into its buffer: not 16-byte
+    aligned, so the pointwise and stencil launchers take their scalar / generic kernels"""
+    import torch
+
+    buf = torch.empty(t.numel() + 1, dtype=t.dtype, device=t.device)
+    v = buf[1:].view(t.shape)
+    v.copy_(t)
+    assert v.data_ptr() % 16 != 0
+    return v
+
+
+def hand_fused_vs_oracle(d8, dem, thr, px=PX, n=0.4, b=0.1, size=None):
+    """fused flow accumulation + HAND (entry_done) on a D8 grid against the oracle, with GFI parameters (n, b, size)
+    (size defaults to px, as example.py:87 passes it); returns the kernel profile"""
     import torch
 
     from descriptools_b200 import _lib, device
 
+    size = px if size is None else size
     acc_ref, _ = oracle.flow_accumulation(d8)
     river = (acc_ref > thr).astype(np.int8)
     f_ref, i_ref, h_ref = oracle.flow_hand_index(dem, d8, river, px)
-    g_ref = oracle.gfi(h_ref, acc_ref, i_ref, 0.4, 0.1, px)
+    with np.errstate(all="ignore"):
+        g_ref = oracle.gfi(h_ref, acc_ref, i_ref, n, b, size)
     t8, td = torch.from_numpy(d8).cuda(), torch.from_numpy(dem).cuda()
     _lib.profile_enable(True)
     try:
         acc = device.flow_accumulation(t8, fuse_hand_threshold=thr)
-        out = device.hand(t8, td, px, acc=acc, river_threshold=thr, gfi_params=(0.4, 0.1, px), entry_done=True)
+        out = device.hand(t8, td, px, acc=acc, river_threshold=thr, gfi_params=(n, b, size), entry_done=True)
         torch.cuda.synchronize()
         prof = _lib.profile_collect()
     finally:

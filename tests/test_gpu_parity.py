@@ -8,7 +8,7 @@ import pytest
 import torch
 
 import oracle
-from helpers import example_inputs, hand_fused_vs_oracle, listed_tiles, load, serpentine_d8, sha, synth
+from helpers import example_inputs, hand_fused_vs_oracle, listed_tiles, load, misaligned, serpentine_d8, sha, synth
 
 pytestmark = pytest.mark.gpu
 
@@ -33,15 +33,6 @@ def ex():
 
 
 # ---- slope + D8 -------------------------------------------------------------------------------
-def misaligned(t):
-    """the same values in a contiguous view that starts 4 bytes into its buffer: not 16-byte aligned"""
-    buf = torch.empty(t.numel() + 1, dtype=t.dtype, device=t.device)
-    v = buf[1:].view(t.shape)
-    v.copy_(t)
-    assert v.data_ptr() % 16 != 0
-    return v
-
-
 def check_slope_d8(mods, dem, px):
     """all three launch forms (slope only, D8 only, both outputs -- the fused kernel of the chain) against the oracle;
     then all three again on a DEM that is not 16-byte aligned, which only the generic kernel takes"""

@@ -137,6 +137,13 @@ SIGNATURES = {
                                 c_void_p, c_size_t, c_void_p]),
     "dtb_eval_class_map": (c_int, [c_void_p, c_int, c_void_p, c_int64, c_double, c_double, c_int, c_void_p, c_void_p, c_void_p]),
     "dtb_minmax_scale": (c_int, [c_void_p, c_int, c_int64, c_double, c_double, c_double, c_void_p, c_void_p]),
+    "dtb_eval_counts_from_hist": (c_int, [c_void_p, c_int, c_int, POINTER(c_int64)]),
+    "dtb_eval_extrema_workspace_bytes": (c_size_t, []),
+    "dtb_eval_extrema": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "dtb_eval_hist": (c_int, [c_void_p, c_int, c_void_p, c_int64, c_double, c_double, c_double, c_double, POINTER(c_double), c_int,
+                              c_int, c_void_p, c_void_p]),
+    "dtb_eval_class_scaled": (c_int, [c_void_p, c_int, c_void_p, c_int64, c_double, c_double, c_double, c_double, c_double, c_int,
+                                      c_void_p, c_void_p]),
     "dtb_tiff_decode_workspace_bytes": (c_size_t, [POINTER(TiffLayout), c_int64]),
     "dtb_tiff_decode_chunks": (c_int, [POINTER(TiffLayout), c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p,
                                        c_size_t, c_void_p, c_void_p]),

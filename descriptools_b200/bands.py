@@ -220,6 +220,9 @@ class Band:
         self.hand_sum = torch.zeros((8, cols), dtype=i64, device=device)
         self.hand_res = torch.zeros((8, cols), dtype=i64, device=device)
         self.ws_fill = None  # depression filling only: allocated by fill_init, freed by fill_release
+        self.flood = None    # benchmark flood map rows (int8), load_flood
+        self.extra = {}      # ti, mti, lnhlh, <descriptor>_class: allocated on first use (log_indices, calibrate)
+        self.slope_rad = None
 
     # views
     @property
@@ -339,7 +342,62 @@ class Band:
                     "dtb_hand(finish)")
 
     def outputs(self) -> dict:
-        return dict(slope=self.slope, d8=self.d8, acc=self.acc, fdist=self.fdist, idx=self.idx, hand=self.hand, gfi=self.gfi)
+        return dict(slope=self.slope, d8=self.d8, acc=self.acc, fdist=self.fdist, idx=self.idx, hand=self.hand, gfi=self.gfi,
+                    **self.extra)
+
+    def _extra(self, name, dtype):
+        if name not in self.extra:
+            self.extra[name] = torch.empty((self.rows, self.cols), dtype=dtype, device=self.dev)
+        return self.extra[name]
+
+    def log_indices(self, n_top: float):
+        """TI and MTI (topoindexes.py:109-167, slope in radians as example.py:63-64 makes it) and ln(hl/H) (gfi.py:297-346,
+        size = px) of the band's rows: pointwise, no exchange"""
+        from ._lib import DTB_I32, DTB_I64
+
+        n = self.rows * self.cols
+        idt = DTB_I64 if self.int_dt == torch.int64 else DTB_I32
+        if self.slope_rad is None:
+            self.slope_rad = torch.empty((self.rows, self.cols), dtype=torch.float32, device=self.dev)
+        rad = self.slope_rad
+        ti, mti, ln = self._extra("ti", torch.float32), self._extra("mti", torch.float32), self._extra("lnhlh", torch.float32)
+        self._check(self.lib.dtb_slope_to_radians(self.slope.data_ptr(), n, rad.data_ptr(), self._stream()), "dtb_slope_to_radians")
+        self._check(self.lib.dtb_ti_mti(self.acc.data_ptr(), idt, rad.data_ptr(), n, self.px, float(n_top), ti.data_ptr(), mti.data_ptr(),
+                                        self._stream()), "dtb_ti_mti")
+        self._check(self.lib.dtb_lnhlh(self.hand.data_ptr(), 0, self.acc.data_ptr(), idt, n, self.n_gfi, self.b_gfi, self.px, ln.data_ptr(),
+                                       self._stream()), "dtb_lnhlh")
+
+    # calibration (calibrate_bands)
+    def _descriptor(self, name):
+        t = self.outputs().get(name)
+        if t is None or t.dtype != torch.float32:
+            raise ValueError(f"{name!r} is not a float32 raster of the bands (calibrate hand, gfi, ti, mti, lnhlh, ...)")
+        if self.flood is None:
+            raise RuntimeError("calibration needs the benchmark flood map: load_flood() first")
+        return t
+
+    def extrema(self, descriptor: str) -> torch.Tensor:
+        """float64 [5]: the band's part of np.unique's two ends (device.eval_extrema)"""
+        from . import device
+
+        return device.eval_extrema(self._descriptor(descriptor))
+
+    def corner(self, descriptor: str) -> torch.Tensor:
+        """float64 [1]: the band's first cell (band 0: the raster's cell (0, 0), binary_map's nodata)"""
+        return self._descriptor(descriptor)[0, :1].to(torch.float64)
+
+    def histogram(self, descriptor, mn, mx, corner, thresholds, under, nodata, hist):
+        """add the band's scaled confusion histogram into hist (device.eval_hist)"""
+        from . import device
+
+        device.eval_hist(self._descriptor(descriptor), self.flood, mn, mx, corner, thresholds, under, hist, nodata)
+
+    def class_map(self, descriptor, mn, mx, corner, threshold, under, nodata):
+        """the band's rows of the class map, kept as `<descriptor>_class` (int8)"""
+        from . import device
+
+        d = self._descriptor(descriptor)
+        device.eval_class(d, self.flood, mn, mx, corner, threshold, under, nodata, out=self._extra(descriptor + "_class", torch.int8))
 
     # depression filling (fill_rounds): the (rows + 2) x cols view dem_buf[1:rows+3], one halo row per side
     def fill_halo_items(self):
@@ -407,6 +465,43 @@ def fill_rounds(bands, x, max_rounds: int = FILL_MAX_ROUNDS) -> dict:
         for b in bands:
             b.fill_release()
     raise RuntimeError(f"depression filling over bands did not converge in {max_rounds} rounds")
+
+
+# ---- calibration over bands --------------------------------------------------------------------------------
+def calibrate_bands(bands, x, descriptor: str = "hand", under: str = "under", nodata: float = -100) -> dict:
+    """Calibrate the raster `descriptor` held by `bands` (this process's bands; `x` the exchange) against the benchmark
+    flood map the bands hold: the numbers device.calibrate gives on the whole raster, and every band's rows of its class
+    map, with no rank holding more than its band.
+
+      1. every band's extrema (two smallest distinct values, largest, NaN seen) are gathered and merged on the host by
+         np.unique's rule (evaluation.unique_ends) -> mn, mx; band 0 broadcasts the raw value of cell (0, 0);
+      2. per stage of the threshold search (evaluation.search_threshold) every band adds its scaled histogram into one
+         buffer, which is summed over the ranks (all_sum) and turned into the stage's counts on the host;
+      3. every band writes its rows of the class map at the threshold found.
+
+    A band is anything with extrema / corner / histogram / class_map (tests pass NumPy stand-ins).
+    Returns {"threshold", "correctness", "fit", "mn", "mx", "counts": (tn, fp, fn, tp)}."""
+    from . import evaluation
+
+    if under not in ("under", "over"):
+        raise ValueError("under must be 'under' or 'over'")
+    ext = x.gather([b.extrema(descriptor) for b in bands])
+    mn, mx = evaluation.unique_ends(ext.cpu().numpy())
+    corner = bands[0].corner(descriptor) if bands[0].index == 0 else torch.zeros(1, dtype=torch.float64, device=ext.device)
+    x.broadcast(corner, 0)
+    corner = float(corner.cpu()[0])
+    hist = torch.zeros(4 * 33, dtype=torch.int64, device=ext.device)
+
+    def counts(thresholds):
+        hist.zero_()
+        for b in bands:
+            b.histogram(descriptor, mn, mx, corner, thresholds, under, nodata, hist)
+        return evaluation.counts_from_hist(x.all_sum(hist).cpu().numpy(), len(thresholds), under)
+
+    th, c, f, cnt = evaluation.search_threshold(counts)
+    for b in bands:
+        b.class_map(descriptor, mn, mx, corner, th, under, nodata)
+    return dict(threshold=th, correctness=c, fit=f, mn=mn, mx=mx, counts=cnt)
 
 
 # ---- raster files from bands -------------------------------------------------------------------------
@@ -639,7 +734,7 @@ class _Exchange:
         """per_band: the summaries of this process's bands.  Every band's summary is gathered here and this process solves
         the (small) boundary graph itself, keeping its own bands' answers: one collective per solve, and no rank waits
         for rank 0 to prepare and scatter."""
-        res, flag = self.graphed(solver, self._gather(per_band), rounds)
+        res, flag = self.graphed(solver, self.gather(per_band), rounds)
         self.flags.append(flag.clone())
         return [res[i].clone() for i in self.local_bands]
 
@@ -670,7 +765,8 @@ class LocalExchange(_Exchange):
     def broadcast(self, t: torch.Tensor, band: int):
         """one process: t already holds band `band`'s rows"""
 
-    def _gather(self, per_band):
+    def gather(self, per_band):
+        """the tensors of every band, stacked in band order"""
         return torch.stack(per_band, 0)
 
 
@@ -723,7 +819,8 @@ class DistExchange(_Exchange):
         """t on every rank := t on the rank holding band `band`"""
         self.dist.broadcast(t, src=self._peer(band), group=self.group)
 
-    def _gather(self, per_band):
+    def gather(self, per_band):
+        """the tensors of every band (one per rank, same shape), stacked in band order on every rank"""
         (mine,), d = per_band, self.dist
         mine = mine.contiguous()
         everyone = torch.empty((self.world,) + tuple(mine.shape), dtype=mine.dtype, device=mine.device)
@@ -810,6 +907,35 @@ class BandRunner:
                 _device.nodata_to_sentinel(b.dem, nd)
         if condition:
             self.fill_depressions()
+
+    def load_flood(self, path):
+        """Every local band reads its rows of a benchmark flood map GeoTIFF (uint8 or int8, the DEM's shape) to its device,
+        kept as int8 (what example.py:106's .astype("int8") makes of it) for calibrate()."""
+        from . import raster
+
+        with raster.open(path) as src:
+            if src.shape != (self.rows, self.cols):
+                raise ValueError(f"{path}: flood map is {src.shape}, the runner was built for {(self.rows, self.cols)}")
+            dt = src.dtypes[0]
+            if dt not in ("uint8", "int8"):
+                raise TypeError(f"{path}: the flood map must be uint8 or int8, the file holds {dt}")
+            for b in self.bands:
+                t = torch.empty((b.rows, self.cols), dtype=getattr(torch, dt), device=b.dev)
+                raster.read_to_device(src, out=t, rows=(b.r0, b.r1))
+                b.flood = t.view(torch.int8)
+
+    def calibrate(self, descriptor: str = "hand", under: str = "under", nodata: float = -100) -> dict:
+        """Calibrate a float32 raster of the bands (after step(); "hand" with "under" as example.py:136 does, "gfi" with
+        "over", or ti / mti / lnhlh after log_indices()) against the flood map of load_flood (calibrate_bands).  The
+        class map becomes the output `<descriptor>_class`.  Returns the threshold, correctness and fit indexes, mn, mx
+        and the counts at the threshold, equal to device.calibrate on the whole raster."""
+        return calibrate_bands(self.bands, self.x, descriptor, under, nodata)
+
+    def log_indices(self, n_top: float = 0.1):
+        """TI and MTI (example.py:63-69) and ln(hl/H) (example.py:91, with the runner's GFI exponent and scale, size = px)
+        of every local band after step(): the outputs `ti`, `mti` and `lnhlh`."""
+        for b in self.bands:
+            b.log_indices(n_top)
 
     def step(self, events=None, hook=None, check=True):
         """One pass of the chain; `events` (4 CUDA events) are recorded at the stage boundaries and `hook(i)` is
@@ -1000,8 +1126,9 @@ class BandRunner:
 
     def write_files(self, out_dir, outputs=None, compress: str = "lzw", blocksize: int = 256, **geo) -> dict:
         """The chain's rasters of the last step() as `out_dir/<name>.tif`, with the metadata pipeline.pipeline_files uses
-        (pipeline.output_meta) and the DEM's georeferencing from load_file (or `geo`): the seven files are byte for byte
-        those pipeline_files writes on one GPU.  Returns {name: path}."""
+        (pipeline.output_meta) and the DEM's georeferencing from load_file (or `geo`): the files are byte for byte those
+        pipeline_files writes on one GPU.  `outputs` defaults to the seven chain rasters; ti, mti, lnhlh (log_indices) and
+        <descriptor>_class (calibrate; uint8, nodata 0, as example.py:205-206 writes it) may be listed.  Returns {name: path}."""
         import os
 
         from .pipeline import STAGE_OUTPUTS, output_meta
@@ -1010,7 +1137,9 @@ class BandRunner:
         paths = {}
         outs = self.outputs()
         for name in (STAGE_OUTPUTS if outputs is None else outputs):
-            per_band = [o[name] for o in outs]
+            if name not in outs[0]:
+                raise ValueError(f"{name!r} is not an output of the bands (log_indices() / calibrate() add ti, mti, lnhlh and *_class)")
+            per_band = [o[name].view(torch.uint8) if name.endswith("_class") else o[name] for o in outs]
             paths[name] = os.path.join(out_dir, name + ".tif")
             self.write_raster(paths[name], per_band, **output_meta(name, per_band[0].dtype.is_floating_point, compress, blocksize), **geo)
         return paths

@@ -300,6 +300,103 @@ def slope_to_radians(slope_pct: torch.Tensor) -> torch.Tensor:
     return out
 
 
+# ---- calibration against a benchmark flood map without the float64 raster (csrc/evaluation.cu) ----------------------
+_EV_DT = {torch.float32: 0, torch.int16: 2}  # DTB_EV_F32, DTB_EV_I16
+
+
+def _ev_dtype(t: torch.Tensor) -> int:
+    try:
+        return _EV_DT[t.dtype]
+    except KeyError:
+        raise TypeError(f"calibrated descriptors must be float32 or int16, got {t.dtype}") from None
+
+
+def flood_int8(flood: torch.Tensor, like: torch.Tensor) -> torch.Tensor:
+    """a benchmark flood map as the kernels read it: int8, or uint8 viewed as int8 (what .astype("int8") makes of it)"""
+    flood = _chk2d(flood, "flood")
+    if flood.dtype == torch.uint8:
+        flood = flood.view(torch.int8)
+    elif flood.dtype != torch.int8:
+        raise TypeError(f"the flood map must be int8 or uint8, got {flood.dtype}")
+    _same_shape(descriptor=like, flood=flood)
+    return flood
+
+
+def eval_extrema(desc: torch.Tensor) -> torch.Tensor:
+    """float64 [5] on the device, no host sync: smallest and second-smallest distinct non-NaN values, largest non-NaN
+    value, distinct non-NaN values seen (capped at 2), NaN seen -- the two ends of np.unique(desc) (dtb_eval_extrema)"""
+    desc = _chk2d(desc, "descriptor")
+    out = torch.empty(5, dtype=torch.float64, device=desc.device)
+    nbytes = lib.dtb_eval_extrema_workspace_bytes()
+    with torch.cuda.device(desc.device):
+        ws = workspace.get(nbytes, "extrema", desc.device)
+        check(lib.dtb_eval_extrema(_ptr(desc), _ev_dtype(desc), desc.numel(), _ptr(out), _ptr(ws), nbytes, _stream()), "dtb_eval_extrema")
+    return out
+
+
+def eval_hist(desc: torch.Tensor, flood: torch.Tensor, mn: float, mx: float, corner: float, thresholds, under: str,
+              hist: torch.Tensor, nodata: float = -100) -> torch.Tensor:
+    """ADD the 4 x 33 confusion histogram of `thresholds` (strictly ascending, at most 32) on minMaxScale(desc, mn, mx,
+    nodata) into `hist` (int64 [4 * 33] on desc's device), scaling every cell on load; `corner` is the raw value of the
+    raster's cell (0, 0), binary_map's nodata after scaling (dtb_eval_hist).  No host sync."""
+    desc = _chk2d(desc, "descriptor")
+    flood = flood_int8(flood, desc)
+    if hist.dtype != torch.int64 or hist.numel() != 4 * 33 or hist.device != desc.device or not hist.is_contiguous():
+        raise ValueError("hist must be a contiguous int64 tensor of 4 x 33 entries on the descriptor's device")
+    th = np.ascontiguousarray(thresholds, dtype=np.float64)
+    with torch.cuda.device(desc.device):
+        check(lib.dtb_eval_hist(_ptr(desc), _ev_dtype(desc), _ptr(flood), desc.numel(), float(mn), float(mx), float(nodata),
+                                float(corner), th.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), len(th),
+                                1 if under == "under" else 0, _ptr(hist), _stream()), "dtb_eval_hist")
+    return hist
+
+
+def eval_class(desc: torch.Tensor, flood: torch.Tensor, mn: float, mx: float, corner: float, threshold: float, under: str,
+               nodata: float = -100, out: torch.Tensor | None = None) -> torch.Tensor:
+    """int8 class map (0 tn, 1 fp, 2 fn, 3 tp) = avaliacao(binary_map(minMaxScale(desc, mn, mx, nodata), threshold), flood),
+    scaled on load like eval_hist (dtb_eval_class_scaled)"""
+    desc = _chk2d(desc, "descriptor")
+    flood = flood_int8(flood, desc)
+    cls = _out(None if out is None else {"cls": out}, "cls", tuple(desc.shape), torch.int8, desc.device)
+    with torch.cuda.device(desc.device):
+        check(lib.dtb_eval_class_scaled(_ptr(desc), _ev_dtype(desc), _ptr(flood), desc.numel(), float(mn), float(mx), float(nodata),
+                                        float(corner), float(threshold), 1 if under == "under" else 0, _ptr(cls), _stream()),
+              "dtb_eval_class_scaled")
+    return cls
+
+
+def calibrate(desc: torch.Tensor, flood: torch.Tensor, under: str = "under", nodata: float = -100) -> dict:
+    """Calibrate a descriptor against a benchmark flood map on the device: what example.py:113-147 does with np.unique,
+    minMaxScale, calibration, binary_map and avaliacao, without the float64 raster and without modifying `flood`.
+
+    desc: float32 or int16 CUDA tensor; flood: int8 or uint8 of the same shape.  One extrema pass gives
+    mn = np.unique(desc)[1] and mx = np.unique(desc)[-1], then one scaled histogram pass per stage of the threshold search
+    (evaluation.search_threshold) and one class-map pass.  Returns {"threshold", "correctness", "fit", "mn", "mx",
+    "counts": (tn, fp, fn, tp) at the threshold, "class_map": int8 CUDA tensor}.  ValueError if desc has fewer than two
+    distinct values."""
+    from . import evaluation
+
+    desc = _chk2d(desc, "descriptor")
+    _ev_dtype(desc)
+    flood = flood_int8(flood, desc)
+    if under not in ("under", "over"):
+        raise ValueError("under must be 'under' or 'over'")
+    with torch.cuda.device(desc.device):
+        ext = torch.cat([eval_extrema(desc), desc.reshape(-1)[:1].to(torch.float64)]).cpu().numpy()
+        mn, mx = evaluation.unique_ends(ext[:5])
+        corner = float(ext[5])
+        hist = torch.empty(4 * 33, dtype=torch.int64, device=desc.device)
+
+        def counts(thresholds):
+            hist.zero_()
+            eval_hist(desc, flood, mn, mx, corner, thresholds, under, hist, nodata)
+            return evaluation.counts_from_hist(hist.cpu().numpy(), len(thresholds), under)
+
+        th, c, f, cnt = evaluation.search_threshold(counts)
+        cls = eval_class(desc, flood, mn, mx, corner, th, under, nodata)
+    return dict(threshold=th, correctness=c, fit=f, mn=mn, mx=mx, counts=cnt, class_map=cls)
+
+
 def chain_check(d8: torch.Tensor, acc: torch.Tensor, river_threshold: int, idx: torch.Tensor | None = None,
                 dem: torch.Tensor | None = None, hand: torch.Tensor | None = None, row0: int = 0,
                 total_rows: int | None = None) -> torch.Tensor:

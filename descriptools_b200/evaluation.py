@@ -71,12 +71,6 @@ class _Counter:
         back[order] = inv
         return out[back]  # row i <-> thresholds[i]: (tn, fp, fn, tp)
 
-    def fits(self, thresholds):
-        c = self.counts(thresholds)
-        # fit index: tp / (tp + fn + fp)  (evaluation.py:192-211); numpy int division like the reference
-        with np.errstate(divide="ignore", invalid="ignore"):
-            return c[:, 3] / (c[:, 3] + c[:, 2] + c[:, 1])
-
 
 def minMaxScale(mat, mn, mx, nodata):
     """evaluation.py:5-9: nodata -> NaN, the rest (mat - mn) / (mx - mn); float64."""
@@ -92,35 +86,83 @@ def minMaxScale(mat, mn, mx, nodata):
     return out.cpu().numpy()
 
 
-def calibration(descriptor_matrix, comparison_matrix, under):
-    """Best threshold for the linear binary classification -- evaluation.py:12-87 (same search, same tie rules).
-    Like the reference it leaves `comparison_matrix` remapped in place (1 -> 2, -100 -> 0)."""
-    d, nodata, is_f64 = _dev_desc(descriptor_matrix)
-    _remap_inplace(comparison_matrix)  # what the first avaliacao call of the reference does (evaluation.py:32)
-    k = _Counter(d, is_f64, nodata, _flood_dev(comparison_matrix), under)
-    f1, f2, f3 = k.fits([25 / 100, 50 / 100, 75 / 100])  # evaluation.py:32-37
+def search_threshold(counts):
+    """The threshold search of calibration (evaluation.py:32-87): five stages of thresholds on the scaled descriptor, the
+    first three in steps of 0.25, then 0.1, 0.01, 0.001 and 0.0001 around the best so far, with the reference's tie rules
+    (the stage-1 pick, `>=` in stage 2, `>` after it).  `counts(thresholds)` -> (len, 4) int64 rows (tn, fp, fn, tp), one
+    call per stage: the drop-in, device.calibrate and the row-band driver differ only in where those counts come from.
+
+    Returns (threshold, correctness index, fit index, (tn, fp, fn, tp)) at the threshold, taken from the last stage's
+    counts: the final threshold is always a member of that stage's list (its centre, if nothing beats it)."""
+    def fits(c):
+        # fit index: tp / (tp + fn + fp)  (evaluation.py:192-211); numpy int division like the reference
+        with np.errstate(divide="ignore", invalid="ignore"):
+            return c[:, 3] / (c[:, 3] + c[:, 2] + c[:, 1])
+
+    f1, f2, f3 = fits(counts([25 / 100, 50 / 100, 75 / 100]))  # evaluation.py:32-37
     if f3 > f2:
         fit_index, iteration_value = (f3, 75) if f3 > f1 else (f1, 25)
     else:
         fit_index, iteration_value = (f2, 50) if f2 > f1 else (f1, 25)
     threshold = None
     steps = list(range(iteration_value - 20, iteration_value + 30, 10))  # evaluation.py:54-59
-    for i, v in zip(steps, k.fits([i / 100 for i in steps])):
+    for i, v in zip(steps, fits(counts([i / 100 for i in steps]))):
         if v >= fit_index:
             fit_index, threshold = v, i
     iteration_value = threshold
     steps = list(range(iteration_value - 5, iteration_value + 6, 1))  # evaluation.py:61-66
-    for i, v in zip(steps, k.fits([i / 100 for i in steps])):
+    for i, v in zip(steps, fits(counts([i / 100 for i in steps]))):
         if v > fit_index:
             fit_index, threshold = v, i
     for scale in (1000, 10000):  # evaluation.py:68-85
         iteration_value = threshold * 10
         threshold = iteration_value
         steps = list(range(iteration_value - 10, iteration_value + 11, 1))
-        for i, v in zip(steps, k.fits([i / scale for i in steps])):
+        last = counts([i / scale for i in steps])
+        for i, v in zip(steps, fits(last)):
             if v > fit_index:
                 fit_index, threshold = v, i
-    return threshold / 10000
+    tn, fp, fn, tp = (int(v) for v in last[steps.index(threshold)])
+    with np.errstate(divide="ignore", invalid="ignore"):
+        correctness_index = np.int64(tp) / np.int64(fn + tp)          # evaluation.py:174-190
+        fit = np.int64(tp) / np.int64(tp + fn + fp)
+    return threshold / 10000, float(correctness_index), float(fit), (tn, fp, fn, tp)
+
+
+def calibration(descriptor_matrix, comparison_matrix, under):
+    """Best threshold for the linear binary classification -- evaluation.py:12-87 (same search, same tie rules).
+    Like the reference it leaves `comparison_matrix` remapped in place (1 -> 2, -100 -> 0)."""
+    d, nodata, is_f64 = _dev_desc(descriptor_matrix)
+    _remap_inplace(comparison_matrix)  # what the first avaliacao call of the reference does (evaluation.py:32)
+    k = _Counter(d, is_f64, nodata, _flood_dev(comparison_matrix), under)
+    return search_threshold(k.counts)[0]
+
+
+def counts_from_hist(hist, k: int, under) -> np.ndarray:
+    """(k, 4) int64 (tn, fp, fn, tp) of the k thresholds a 4 x 33 histogram of dtb_eval_hist was taken for (host only)"""
+    h = np.ascontiguousarray(np.asarray(hist).reshape(-1), dtype=np.int64)
+    if h.size != 4 * 33:
+        raise ValueError("a calibration histogram has 4 x 33 entries")
+    out = np.zeros((k, 4), np.int64)
+    check(lib.dtb_eval_counts_from_hist(h.ctypes.data, int(k), 1 if under == "under" else 0,
+                                        out.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))), "dtb_eval_counts_from_hist")
+    return out
+
+
+def unique_ends(extrema):
+    """(mn, mx) = (np.unique(x)[1], np.unique(x)[-1]) (example.py:113-115) from the extrema rows of the parts of x (rows of
+    dtb_eval_extrema: lo, second lo, hi, distinct non-NaN values capped at 2, NaN seen).  np.unique keeps one NaN and sorts
+    it last, so a NaN anywhere makes mx NaN, and mn is NaN when only one non-NaN value exists.  Fewer than two values
+    raise ValueError (the reference's IndexError at elements[1])."""
+    e = np.asarray(extrema, dtype=np.float64).reshape(-1, 5)
+    cnt = e[:, 3].astype(np.int64)
+    small = np.unique(np.concatenate([e[cnt >= 1, 0], e[cnt >= 2, 1]]))[:2]  # two smallest distinct values of the union
+    has_nan = bool((e[:, 4] != 0).any())
+    if len(small) + has_nan < 2:
+        raise ValueError("the descriptor has fewer than two distinct values: np.unique(descriptor)[1] does not exist")
+    mn = small[1] if len(small) >= 2 else np.nan
+    mx = np.nan if has_nan else e[cnt >= 1, 2].max()
+    return float(mn), float(mx)
 
 
 def binary_map(descriptor_matrix, threshold, under):

@@ -20,6 +20,7 @@ from . import device
 from ._convert import dem_to_native
 
 STAGE_OUTPUTS = ("slope", "d8", "acc", "fdist", "idx", "hand", "gfi")
+LOG_OUTPUTS = ("ti", "mti", "lnhlh")  # pipeline_files(outputs=...) and BandRunner.log_indices
 
 
 def alloc_outputs(rows: int, cols: int, dem_dtype: torch.dtype = torch.float32, device=None) -> dict:
@@ -152,15 +153,16 @@ def output_dtypes(dem_dtype: np.dtype, n_cells: int) -> dict:
 
 def output_meta(name: str, floating: bool, compress: str = "lzw", blocksize: int = 256) -> dict:
     """file metadata of the chain's raster `name` (pipeline_files, bands.BandRunner.write_files): tiled, the predictor that
-    suits the samples (3 floating point, 2 integers), nodata -100 (0 for the D8 codes, like 12_fdr.tif)"""
+    suits the samples (3 floating point, 2 integers), nodata -100 (0 for the D8 codes, like 12_fdr.tif, and for class
+    maps, like example.py:206)"""
     return dict(compress=compress, predictor=1 if compress in (None, "none") else (3 if floating else 2), tiled=True, blockxsize=blocksize,
-                blockysize=blocksize, nodata=0 if name == "d8" else -100)
+                blockysize=blocksize, nodata=0 if name == "d8" or name.endswith("_class") else -100)
 
 
 def pipeline_files(dem_path, out_dir, river_threshold: int, px: float | None = None, n_gfi: float = 0.4,
                    scale_factor: float = 0.1, size: float | None = None, outputs=STAGE_OUTPUTS, compress: str = "lzw",
                    blocksize: int = 256, block_bytes: int = 256 << 20, threads: int = 0, decode: str = "auto", encode: str = "auto",
-                   condition: bool = False) -> dict:
+                   condition: bool = False, flood=None, under: str = "under", n_top: float = 0.1) -> dict:
     """The chain from a DEM GeoTIFF to one GeoTIFF per descriptor (`out_dir/<name>.tif`), what a user of the
     reference does around the descriptor calls with rasterio (example.py:33, :42-43, :201-217).
 
@@ -174,13 +176,22 @@ def pipeline_files(dem_path, out_dir, river_threshold: int, px: float | None = N
     for DEMs that no GIS has conditioned yet (float32 only).
     `decode` / `encode`: "device", "host", or "auto" (default) = the device codec whenever it can take the file
     (stored or LZW chunks), the host codec for the rest (Deflate, PackBits, chunks over 1 MiB).
-    Returns {name: path}.
+    `outputs` may also list "ti", "mti" (example.py:63-69, exponent `n_top`), "lnhlh" (example.py:91) and, with a
+    benchmark flood map GeoTIFF `flood` (uint8 / int8, the DEM's shape), "hand_class": HAND calibrated against it
+    (device.calibrate, direction `under`; example.py:113-147), written as uint8 with nodata 0 (example.py:201-217).
+    Returns {name: path}, plus "calibration": the numbers of device.calibrate when `flood` is given.
     """
     import torch
 
     from . import raster
 
     device.require_cuda()
+    known = STAGE_OUTPUTS + LOG_OUTPUTS + ("hand_class",)
+    for name in outputs:
+        if name not in known:
+            raise ValueError(f"unknown output {name!r} (one of {', '.join(known)})")
+    if "hand_class" in outputs and flood is None:
+        raise ValueError("the output 'hand_class' needs a benchmark flood map (flood=...)")
     with raster.open(dem_path) as src:
         geo = dict(crs=src.crs, transform=src.transform)
         if px is None:
@@ -199,6 +210,17 @@ def pipeline_files(dem_path, out_dir, river_threshold: int, px: float | None = N
             raise TypeError("condition=True needs a float32 DEM (the filling raises cells by single float32 steps)")
         device.fill_depressions(dem)
     res = run_device(dem, float(px), int(river_threshold), n_gfi, scale_factor, size)
+    if any(name in outputs for name in ("ti", "mti")):
+        res["ti"], res["mti"] = device.ti_mti(res["acc"], device.slope_to_radians(res["slope"]), float(px), n_top)
+    if "lnhlh" in outputs:
+        res["lnhlh"] = device.ln_hl_H(res["hand"], res["acc"], n_gfi, scale_factor, px if size is None else size)
+    calib = None
+    if flood is not None:
+        fl = raster.read_to_device(flood, block_bytes=block_bytes, threads=threads, decode=decode)
+        if tuple(fl.shape) != tuple(dem.shape):
+            raise ValueError(f"{flood}: flood map is {tuple(fl.shape)}, the DEM {tuple(dem.shape)}")
+        calib = device.calibrate(res["hand"], fl, under)
+        res["hand_class"] = calib.pop("class_map").view(torch.uint8)
     os.makedirs(out_dir, exist_ok=True)
     paths = {}
     for name in outputs:
@@ -206,4 +228,6 @@ def pipeline_files(dem_path, out_dir, river_threshold: int, px: float | None = N
         paths[name] = os.path.join(out_dir, name + ".tif")
         raster.write_from_device(paths[name], t, block_bytes=block_bytes, threads=threads, encode=encode,
                                  **output_meta(name, t.dtype.is_floating_point, compress, blocksize), **geo)
+    if calib is not None:
+        paths["calibration"] = calib
     return paths

@@ -299,6 +299,30 @@ int dtb_eval_class_map(const void *desc, int desc_is_f64, const int8_t *flood, i
                        double threshold, int under, int8_t *binary, int8_t *cls, void *stream);
 int dtb_minmax_scale(const void *mat, int mat_dtype, int64_t n, double mn, double mx, double nodata,
                      double *out, void *stream);
+/* dtb_eval_counts_from_hist (host only): the prefix sums that turn a histogram into the counts of dtb_eval_counts.
+ *   hist_host: 4 x 33 uint64, hist[c * 33 + j] = cells of avaliacao class c (0..3, the remapped benchmark) for which
+ *   exactly j of the k thresholds do not flag the cell before the first one that does (under: j = #{th < d}, over:
+ *   j = #{th <= d}; never-flagged cells at j = k under, j = 0 over); counts_host: k x 4 (tn, fp, fn, tp).
+ *
+ * Calibration without the float64 raster of minMaxScale (a descriptor on the device, or one row band of it):
+ * dtb_eval_extrema: the two ends of np.unique(desc) in one pass, no host sync.  desc f32 / i16 (DTB_EV_F32 / DTB_EV_I16);
+ *   out (device, 5 doubles) = smallest and second-smallest DISTINCT non-NaN values, largest non-NaN value, number of
+ *   distinct non-NaN values capped at 2 (entries past it are 0), 1 if a NaN occurs.  +0 and -0 are one value (stored as
+ *   +0), +-inf are ordinary values.  ws >= dtb_eval_extrema_workspace_bytes().
+ * dtb_eval_hist: the histogram above for desc f32 / i16 scaled on load: cell v becomes
+ *   (v == nodata || v != v) ? NaN : (v - mn) / (mx - mn) in f64 -- exactly dtb_minmax_scale's value -- and binary_map's
+ *   nodata is the scaled value of `corner`, the RAW value of the raster's cell (0, 0).  ADDS into hist (device, 4 x 33
+ *   uint64, zeroed by the caller): row bands of one raster may add into one buffer.  Thresholds as for dtb_eval_counts.
+ *   No host sync.
+ * dtb_eval_class_scaled: the class map (int8: 0 tn, 1 fp, 2 fn, 3 tp after avaliacao's remapping of the benchmark) of
+ *   one threshold with the same scaling: avaliacao(binary_map(minMaxScale(desc), threshold), flood). */
+int dtb_eval_counts_from_hist(const unsigned long long *hist_host, int k, int under, int64_t *counts_host);
+size_t dtb_eval_extrema_workspace_bytes(void);
+int dtb_eval_extrema(const void *desc, int desc_dtype, int64_t n, double *out, void *ws, size_t ws_bytes, void *stream);
+int dtb_eval_hist(const void *desc, int desc_dtype, const int8_t *flood, int64_t n, double mn, double mx, double nodata,
+                  double corner, const double *thresholds_host, int k, int under, unsigned long long *hist, void *stream);
+int dtb_eval_class_scaled(const void *desc, int desc_dtype, const int8_t *flood, int64_t n, double mn, double mx,
+                          double nodata, double corner, double threshold, int under, int8_t *cls, void *stream);
 
 /* ---- raster files: GeoTIFF chunks decoded on the device (SURVEY.md section 8 f3) ---------
  * Replaces the pixel decode inside rasterio's `rio.open(p).read(1)` (Example/example.py:33-39) for tiled or

@@ -159,6 +159,9 @@ SIGNATURES = {
                                   c_float, c_void_p, c_void_p]),
     "dtb_fill_workspace_bytes": (c_size_t, [c_int64, c_int64]),
     "dtb_fill_depressions_f32": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_size_t, POINTER(c_int), c_void_p]),
+    "dtb_fill_flat_f32": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_size_t, POINTER(c_int), c_void_p]),
+    "dtb_resolve_flats_workspace_bytes": (c_size_t, [c_int64, c_int64]),
+    "dtb_resolve_flats": (c_int, [c_void_p, c_int, c_void_p, c_int64, c_int64, c_void_p, c_size_t, POINTER(c_int64), c_void_p]),
     "dtb_fill_band_workspace_bytes": (c_size_t, [c_int64, c_int64]),
     "dtb_fill_band_f32": (c_int, [c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_void_p, c_size_t, POINTER(c_int), POINTER(c_int),
                                   c_void_p]),

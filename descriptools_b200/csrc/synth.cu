@@ -14,6 +14,11 @@
 //    with W = z on seed cells (raster edge / next to nodata).  Start from an upper bound
 //    (column and row scans U(c) = max(z(c), succ(U(prev)))), then relax tiles in shared memory
 //    (TILE_ITERS sweeps per pass) until a pass changes nothing.
+//  * dtb_fill_flat_f32: the same with succ(m) replaced by m -- the priority flood without epsilon,
+//    which leaves filled areas exactly flat (csrc/flats.cu then gives them D8 codes).  The scans'
+//    bound is above the epsilon fill, so above this one too; relaxing from above ends at the flood
+//    level (every fixed point at or above it equals it), using only min and max: an int16 DEM
+//    filled through a float32 copy is exact.
 #include "common.cuh"
 
 namespace dtb {
@@ -150,7 +155,8 @@ constexpr int TILE_ITERS = 24;  // in-tile sweeps per pass
 // One pass over one tile.  BAND: w points at row 0 of a band whose halo rows -1 / rows (the neighbours' current
 // seam rows) are read where the band has a neighbour -- as constants, never stored -- and *seam is set when a cell
 // of the band's first or last row is lowered.  The single-raster instantiation is the original kernel body.
-template <bool BAND>
+// EPS = false: the fill without epsilon (W = max(z, m) instead of max(z, succ(m))).
+template <bool BAND, bool EPS = true>
 __device__ __forceinline__ void fill_relax_tile(const float *__restrict__ zsrc, const uint8_t *__restrict__ fixed, int64_t rows,
                                                 int64_t cols, float *w, int tiles_x, unsigned *__restrict__ changed,
                                                 int64_t row_lo, int64_t row_hi, unsigned *__restrict__ seam)
@@ -188,7 +194,7 @@ __device__ __forceinline__ void fill_relax_tile(const float *__restrict__ zsrc, 
             const int j = ly + 8 * i + 1, k = lx + 1;
             float m = fminf(fminf(sw[j - 1][k - 1], sw[j - 1][k]), fminf(sw[j - 1][k + 1], sw[j][k - 1]));
             m = fminf(m, fminf(fminf(sw[j][k + 1], sw[j + 1][k - 1]), fminf(sw[j + 1][k], sw[j + 1][k + 1])));
-            const float v = fmaxf(z[i], succ(m));
+            const float v = fmaxf(z[i], EPS ? succ(m) : m);
             if (v < sw[j][k]) {
                 sw[j][k] = v;
                 ch = true;
@@ -217,6 +223,13 @@ fill_relax_kernel(const float *__restrict__ zsrc, const uint8_t *__restrict__ fi
                   float *w, int tiles_x, unsigned *__restrict__ changed)
 {
     fill_relax_tile<false>(zsrc, fixed, rows, cols, w, tiles_x, changed, 0, 0, nullptr);
+}
+
+__global__ void __launch_bounds__(256)
+fill_relax_flat_kernel(const float *__restrict__ zsrc, const uint8_t *__restrict__ fixed, int64_t rows, int64_t cols,
+                       float *w, int tiles_x, unsigned *__restrict__ changed)
+{
+    fill_relax_tile<false, false>(zsrc, fixed, rows, cols, w, tiles_x, changed, 0, 0, nullptr);
 }
 
 // ---- depression filling over row bands ----------------------------------------------------------
@@ -287,8 +300,11 @@ extern "C" size_t dtb_fill_workspace_bytes(int64_t rows, int64_t cols)
     return n * 4 + ((n + 255) / 256) * 256 + 256;
 }
 
-extern "C" int dtb_fill_depressions_f32(float *dem, int64_t rows, int64_t cols, void *ws, size_t ws_bytes,
-                                        int *iterations_host, void *stream)
+namespace {
+// mask, the two upper-bound scans, then relaxation passes of `relax` until one changes nothing
+template <typename Relax>
+int fill_whole(float *dem, int64_t rows, int64_t cols, void *ws, size_t ws_bytes, int *iterations_host, void *stream, Relax relax,
+               const char *relax_name)
 {
     if (!dem || !ws || rows <= 0 || cols <= 0) return DTB_ERR_INVALID;
     if (ws_bytes < dtb_fill_workspace_bytes(rows, cols)) return DTB_ERR_WORKSPACE;
@@ -313,8 +329,8 @@ extern "C" int dtb_fill_depressions_f32(float *dem, int64_t rows, int64_t cols, 
         DTB_CUDA(cudaMemsetAsync(changed, 0, 4, st));
         const int burst = passes < 64 ? 4 : 16;  // check the flag every `burst` passes
         for (int b = 0; b < burst; ++b) {
-            fill_relax_kernel<<<(unsigned)ntiles, 256, 0, st>>>(zsrc, fixed, rows, cols, dem, tiles_x, changed);
-            DTB_LAUNCH_CHECK("fill_relax_kernel");
+            relax<<<(unsigned)ntiles, 256, 0, st>>>(zsrc, fixed, rows, cols, dem, tiles_x, changed);
+            DTB_LAUNCH_CHECK(relax_name);
         }
         passes += burst;
         unsigned h = 0;
@@ -325,6 +341,19 @@ extern "C" int dtb_fill_depressions_f32(float *dem, int64_t rows, int64_t cols, 
     }
     if (iterations_host) *iterations_host = passes;
     return DTB_OK;
+}
+}  // namespace
+
+extern "C" int dtb_fill_depressions_f32(float *dem, int64_t rows, int64_t cols, void *ws, size_t ws_bytes,
+                                        int *iterations_host, void *stream)
+{
+    return fill_whole(dem, rows, cols, ws, ws_bytes, iterations_host, stream, fill_relax_kernel, "fill_relax_kernel");
+}
+
+extern "C" int dtb_fill_flat_f32(float *dem, int64_t rows, int64_t cols, void *ws, size_t ws_bytes, int *iterations_host,
+                                 void *stream)
+{
+    return fill_whole(dem, rows, cols, ws, ws_bytes, iterations_host, stream, fill_relax_flat_kernel, "fill_relax_flat_kernel");
 }
 
 // workspace layout as dtb_fill_workspace_bytes: flags (changed at byte 0, seam at byte 4), zsrc, fixed

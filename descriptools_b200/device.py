@@ -442,18 +442,46 @@ def synth_dem(rows: int, cols: int, row0: int = 0, seed: int = SYNTH_SEED) -> to
     return out
 
 
-def fill_depressions(dem: torch.Tensor) -> int:
-    """In-place priority-flood+epsilon fixed point; returns the number of relaxation passes."""
+def fill_depressions(dem: torch.Tensor, epsilon: bool = True) -> int:
+    """In-place depression filling; returns the number of relaxation passes.
+
+    epsilon=True (float32 only): priority-flood + epsilon, every filled or flat cell raised one float32 step above the
+    neighbour it drains to.  epsilon=False: the priority flood without epsilon, which leaves filled areas exactly flat
+    (give them D8 codes with resolve_flats); float32 or int16 (filled exactly through a float32 copy)."""
     dem_c = _chk2d(dem, "dem")
-    if dem_c.data_ptr() != dem.data_ptr() or dem.dtype != torch.float32:
-        raise ValueError("dem must be a contiguous float32 CUDA tensor")
+    allowed = (torch.float32,) if epsilon else (torch.float32, torch.int16)
+    if dem_c.data_ptr() != dem.data_ptr() or dem.dtype not in allowed:
+        raise ValueError("dem must be a contiguous " + " or ".join(str(t).replace("torch.", "") for t in allowed) + " CUDA tensor")
     rows, cols = dem.shape
     nbytes = lib.dtb_fill_workspace_bytes(rows, cols)
-    ws = workspace.get(nbytes, "fill")
     it = ctypes.c_int(0)
-    check(lib.dtb_fill_depressions_f32(_ptr(dem), rows, cols, _ptr(ws), nbytes, ctypes.byref(it), _stream()),
-          "dtb_fill_depressions_f32")
+    with torch.cuda.device(dem.device):
+        ws = workspace.get(nbytes, "fill", dem.device)
+        work = dem if dem.dtype == torch.float32 else dem.to(torch.float32)
+        fn, name = (lib.dtb_fill_depressions_f32, "dtb_fill_depressions_f32") if epsilon else (lib.dtb_fill_flat_f32, "dtb_fill_flat_f32")
+        check(fn(_ptr(work), rows, cols, _ptr(ws), nbytes, ctypes.byref(it), _stream()), name)
+        if work is not dem:
+            dem.copy_(work)  # every filled value is an elevation of the DEM: exact in int16
     return int(it.value)
+
+
+def resolve_flats(dem: torch.Tensor, d8: torch.Tensor) -> int:
+    """Give D8 codes to the flat cells of `dem` (valid cells whose code in `d8` is 0), in place in `d8`: each flat drains
+    towards its outlets and away from the higher ground around it, and every path ends at an outlet (csrc/flats.cu).
+    The DEM and all other codes are unchanged.  `d8` is slope_d8's output for `dem` (float32 or int16).  Returns the
+    number of cells in flats without an outlet (undrained pits: the DEM was not filled), which keep code 0."""
+    dem, d8_c = _chk2d(dem, "dem"), _chk2d(d8, "d8")
+    if d8.dtype != torch.uint8 or d8_c.data_ptr() != d8.data_ptr():
+        raise ValueError("d8 must be a contiguous uint8 CUDA tensor (it is updated in place)")
+    _same_shape(dem=dem, d8=d8)
+    rows, cols = dem.shape
+    nbytes = lib.dtb_resolve_flats_workspace_bytes(rows, cols)
+    left = ctypes.c_int64(0)
+    with torch.cuda.device(dem.device):
+        ws = workspace.get(nbytes, "flats", dem.device)
+        check(lib.dtb_resolve_flats(_ptr(dem), _dem_dtype(dem), _ptr(d8), rows, cols, _ptr(ws), nbytes, ctypes.byref(left), _stream()),
+              "dtb_resolve_flats")
+    return int(left.value)
 
 
 def conditioned_dem(rows: int, cols: int, seed: int = SYNTH_SEED) -> torch.Tensor:

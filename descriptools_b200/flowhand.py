@@ -71,16 +71,27 @@ def flow_accumulation(flow_direction, nodata=-100):
     return to_host(device.flow_accumulation(to_dev(fdr), dtype=dt, nodata_fill=nodata)).astype(np.int64)
 
 
-def fill_depressions(dem):
+def fill_depressions(dem, epsilon=True):
     """Hydrological conditioning (SURVEY.md section 8 f4): every cell is raised to the lowest level from which water can
-    leave the raster (or reach a nodata cell) along a strictly descending path -- priority-flood + epsilon, the epsilon
-    being one float32 step.  The reference's fixtures were conditioned by an external GIS before example.py:33-39 reads
-    them; an unconditioned DEM leaves interior pits, where D8 has no code and the accumulation stops.  float32 in (other
-    dtypes are converted if exact), float32 out; -100 / NaN cells stay as they are."""
+    leave the raster (or reach a nodata cell).  epsilon=True: priority-flood + epsilon, every filled or flat cell one
+    float32 step above the cell it drains to, so D8 drains it.  The reference's fixtures were conditioned by an external
+    GIS before example.py:33-39 reads them; an unconditioned DEM leaves interior pits, where D8 has no code and the
+    accumulation stops.  float32 in (other dtypes are converted if exact), float32 out.
+    epsilon=False: the priority flood alone; filled areas stay exactly flat (give them codes with resolve_flats).  An
+    int16 DEM stays int16.  -100 / NaN cells stay as they are."""
     d = dem_to_native(dem)
-    if d.dtype != np.float32:
+    if d.dtype != np.float32 and (epsilon or d.dtype != np.int16):
         d = d.astype(np.float32)  # int16 elevations: exact
     t = to_dev(d).clone()
-    device.fill_depressions(t)
+    device.fill_depressions(t, epsilon=epsilon)
     return to_host(t)
 
+
+def resolve_flats(dem, flow_direction):
+    """D8 codes for the flat cells (valid cells with code 0) of `flow_direction`, the D8 raster of `dem`
+    (flow_direction_d8): each flat drains towards its outlets and away from the higher ground around it (Garbrecht &
+    Martz 1997; Barnes, Lehman & Mulla 2014).  Returns a new uint8 raster; the DEM and every other code are unchanged.
+    Flats without an outlet (pits of an unfilled DEM) keep code 0."""
+    t = to_dev(fdr_to_u8(flow_direction)).clone()
+    device.resolve_flats(to_dev(dem_to_native(dem)), t)
+    return to_host(t)

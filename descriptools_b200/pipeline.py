@@ -32,16 +32,19 @@ def alloc_outputs(rows: int, cols: int, dem_dtype: torch.dtype = torch.float32, 
 
 
 def run_device(dem: torch.Tensor, px: float, river_threshold: int, n_gfi: float = 0.4, scale_factor: float = 0.1,
-               size: float | None = None, max_moves: int = 0, out: dict | None = None) -> dict:
+               size: float | None = None, max_moves: int = 0, out: dict | None = None, resolve_flats: bool = False) -> dict:
     """slope(%) f32, d8 u8, acc i32/i64, fdist f32, idx i32/i64, hand (DEM dtype), gfi f32.
 
     river cells are `acc > river_threshold` (example.py:52); GFI uses `size` = px by default
-    (example.py:87).  All tensors stay on the device.
+    (example.py:87).  All tensors stay on the device.  resolve_flats=True gives the flat cells of the DEM D8 codes
+    (device.resolve_flats) before the accumulation -- for a DEM filled with fill_depressions(epsilon=False).
     """
     size = px if size is None else size
     rows, cols = dem.shape
     int_dt = torch.int32 if rows * cols < 2**31 else torch.int64
     slope, d8 = device.slope_d8(dem, px, out=out)
+    if resolve_flats:
+        device.resolve_flats(dem, d8)
     # the last tile pass of the accumulation also does HAND's entry-node pass (river = acc > threshold)
     acc = device.flow_accumulation(d8, dtype=int_dt, nodata_fill=-100, fuse_hand_threshold=river_threshold, out=out)
     out = device.hand(d8, dem, px, acc=acc, river_threshold=river_threshold, max_moves=max_moves,
@@ -162,7 +165,7 @@ def output_meta(name: str, floating: bool, compress: str = "lzw", blocksize: int
 def pipeline_files(dem_path, out_dir, river_threshold: int, px: float | None = None, n_gfi: float = 0.4,
                    scale_factor: float = 0.1, size: float | None = None, outputs=STAGE_OUTPUTS, compress: str = "lzw",
                    blocksize: int = 256, block_bytes: int = 256 << 20, threads: int = 0, decode: str = "auto", encode: str = "auto",
-                   condition: bool = False, flood=None, under: str = "under", n_top: float = 0.1) -> dict:
+                   condition: bool | str = False, flood=None, under: str = "under", n_top: float = 0.1) -> dict:
     """The chain from a DEM GeoTIFF to one GeoTIFF per descriptor (`out_dir/<name>.tif`), what a user of the
     reference does around the descriptor calls with rasterio (example.py:33, :42-43, :201-217).
 
@@ -173,7 +176,9 @@ def pipeline_files(dem_path, out_dir, river_threshold: int, px: float | None = N
     tiles on the GPU and copies only the compressed bytes), tiled and compressed,
     with the DEM's georeferencing; nodata is -100 (0 for the D8 codes, like 12_fdr.tif).
     `condition=True` fills the DEM's depressions on the device first (device.fill_depressions, SURVEY section 8 f4) --
-    for DEMs that no GIS has conditioned yet (float32 only).
+    for DEMs that no GIS has conditioned yet (float32 only).  `condition="flats"` fills them without raising any cell
+    above its flood level (device.fill_depressions(epsilon=False)) and gives the flats D8 codes that drain them
+    (run_device(resolve_flats=True)), so HAND subtracts the DEM's own elevations; float32 and int16.
     `decode` / `encode`: "device", "host", or "auto" (default) = the device codec whenever it can take the file
     (stored or LZW chunks), the host codec for the rest (Deflate, PackBits, chunks over 1 MiB).
     `outputs` may also list "ti", "mti" (example.py:63-69, exponent `n_top`), "lnhlh" (example.py:91) and, with a
@@ -205,11 +210,16 @@ def pipeline_files(dem_path, out_dir, river_threshold: int, px: float | None = N
         device.nodata_to_sentinel(dem, nodata)  # example.py:42-43, one pass (dtb_nodata_to_sentinel_f32)
     elif nodata is not None:
         dem.masked_fill_(dem == nodata, -100)   # int16 DEMs: plumbing only
-    if condition:
+    if condition not in (False, True, "flats"):
+        raise ValueError(f"condition must be False, True or 'flats', got {condition!r}")
+    if condition == "flats":
+        device.fill_depressions(dem, epsilon=False)
+    elif condition:
         if dem.dtype != torch.float32:
-            raise TypeError("condition=True needs a float32 DEM (the filling raises cells by single float32 steps)")
+            raise TypeError("condition=True needs a float32 DEM (the filling raises cells by single float32 steps); "
+                            "condition='flats' takes int16")
         device.fill_depressions(dem)
-    res = run_device(dem, float(px), int(river_threshold), n_gfi, scale_factor, size)
+    res = run_device(dem, float(px), int(river_threshold), n_gfi, scale_factor, size, resolve_flats=condition == "flats")
     if any(name in outputs for name in ("ti", "mti")):
         res["ti"], res["mti"] = device.ti_mti(res["acc"], device.slope_to_radians(res["slope"]), float(px), n_top)
     if "lnhlh" in outputs:

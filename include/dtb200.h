@@ -398,6 +398,26 @@ int dtb_synth_dem_f32(int64_t rows, int64_t cols, int64_t row0, uint32_t seed,
 size_t dtb_fill_workspace_bytes(int64_t rows, int64_t cols);
 int dtb_fill_depressions_f32(float *dem, int64_t rows, int64_t cols, void *ws, size_t ws_bytes,
                              int *iterations_host, void *stream);
+/* The fill without epsilon, same contract and workspace: the fixed point of W = max(z, min over the
+ * neighbours of W) with W = z on the seeds, i.e. a priority flood that leaves filled areas exactly
+ * flat (follow with dtb_resolve_flats).  Uses only min and max, so int16 elevations filled through a
+ * float32 copy stay exact. */
+int dtb_fill_flat_f32(float *dem, int64_t rows, int64_t cols, void *ws, size_t ws_bytes,
+                      int *iterations_host, void *stream);
+
+/* ---- flat resolution (csrc/flats.cu) ----------------------------------------------------------
+ * Gives D8 codes to the flat cells of `dem` (valid cells whose code in d8 is 0; d8 is meant to be
+ * dtb_slope_d8's output for the same DEM, but any D8 raster is read within the raster's bounds), in place: each flat with an outlet (a cell with a code at the flat's elevation
+ * next to it) drains towards its outlets and away from the higher ground around it (Garbrecht &
+ * Martz 1997; Barnes, Lehman & Mulla 2014), every path ending at an outlet.  The DEM, and every code
+ * that is not 0, are not changed.  Flats without an outlet keep code 0; *unresolved_host (may be
+ * NULL) receives their number of cells.  dem_dtype DTB_F32 or DTB_I16; rows * cols < 2^31
+ * (DTB_ERR_UNSUPPORTED otherwise, as is a field that needs more than 200000 passes).  ws: at least
+ * dtb_resolve_flats_workspace_bytes (16 bytes per cell + 4 per 32 x 32 tile + 256).  Synchronous.
+ * When d8 has no flat cell this is one pass over the codes. */
+size_t dtb_resolve_flats_workspace_bytes(int64_t rows, int64_t cols);
+int dtb_resolve_flats(const void *dem, int dem_dtype, uint8_t *d8, int64_t rows, int64_t cols,
+                      void *ws, size_t ws_bytes, int64_t *unresolved_host, void *stream);
 
 /* The same fill over row bands (block-Jacobi: the result equals dtb_fill_depressions_f32 on the
  * whole raster, bit for bit).  dem_halo is (rows + 2) x cols: row 0 and row rows + 1 are halo rows
